@@ -2,6 +2,7 @@
 """bench.py -- throughput of the ALAC packet-decode hot path on B200 (one JSON line on stdout).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c3] [--only-main]
+                    [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over the whole batch. The headline workload is BASELINE configs[2] -- the largest
 config that fits one GPU: 24-bit stereo 192 kHz with bytesShifted=1, 1 h, 168 750 packets of 4096 frames. With --gpus N
@@ -22,8 +23,19 @@ the line reports the max over ranks.
   e2e_api     (N=1) what a caller of the drop-in API pays, through the compiled C++ mirror of the Go package:
               PacketDecoder::DecodePackets over all of c2, NewDecoder + Read over the c1 M4A
 
-Streams come from the test-side encoder on the seeded SURVEY.md section 8d signal (cached under /tmp). The in-run gate
-checks 64 packets per workload against the oracle before timing; the full-size bit-exact checks live in tests/.
+Streams come from the test-side encoder on the seeded SURVEY.md section 8d signal (cached in a per-user temporary
+directory, $ALAC_B200_CACHE to override). The in-run gate checks 64 packets per workload against the oracle before timing;
+the full-size bit-exact checks live in tests/.
+
+--dump-outputs DIR writes what the timed path of the headline workload returned in its last step, so that two builds can
+be compared output for output (the inputs are the same seeded streams from run to run):
+  pcm.npy          float32 [k, frame_length, channels] decoded samples of a fixed seeded sample of k packets (float64 for
+                   32-bit streams; samples past a packet's out_bytes are 0), at most ~56 MB
+  pcm_packets.npy  float64 [k] the indices of those packets in the batch (the first and the short last one included)
+  out_bytes.npy    float64 [n] PCM bytes of every packet
+  status.npy       float64 [n] status word of every packet
+With --gpus N the shards are gathered on rank 0, so the files do not depend on N; --impl reference writes the same files
+from the CPU oracle.
 """
 import argparse
 import ctypes as C
@@ -31,6 +43,7 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -65,13 +78,14 @@ def host_cores():
 
 
 def _cache_dir():
-    d = os.environ.get('ALAC_B200_CACHE', '/tmp/alac_b200_cache')
+    # per user: a cache directory another user created first would not be writable
+    d = os.environ.get('ALAC_B200_CACHE') or os.path.join(tempfile.gettempdir(), f'alac_b200_cache_{os.getuid()}')
     os.makedirs(d, exist_ok=True)
     return d
 
 
 def encode_track(bits, ch, rate, frames, seed, threads, kind='bench', tag=None):
-    """-> (packed u8, offsets u64, sizes u32) of one track from the test-side encoder; cached in /tmp."""
+    """-> (packed u8, offsets u64, sizes u32) of one track from the test-side encoder; cached in _cache_dir()."""
     import oracle_lib as ol
     from signals import make_signal
     path = os.path.join(_cache_dir(), f'{tag or "t"}_{bits}_{ch}_{rate}_{frames}_{kind}_seed{seed}_v1.npz')
@@ -102,7 +116,7 @@ def encode_track(bits, ch, rate, frames, seed, threads, kind='bench', tag=None):
 
 
 def build_workload(name, seed, threads):
-    """-> dict(cfg, cookie, packed u8, offsets u64, sizes u32, frames, channels, bits, rate). Cached in /tmp."""
+    """-> dict(cfg, cookie, packed u8, offsets u64, sizes u32, frames, channels, bits, rate). Cached in _cache_dir()."""
     import oracle_lib as ol
     bits, ch, rate, seconds, _ = WORKLOADS[name]
     cfg = ol.Config.make(bit_depth=bits, num_channels=ch, sample_rate=rate)
@@ -256,6 +270,37 @@ def emit_line(line):
 
 _REAL_STDOUT = 1
 
+DUMP_BYTES = 56 << 20  # everything --dump-outputs writes stays under 64 MB
+
+
+def dump_dtype(bits):
+    return np.float32 if bits <= 24 else np.float64  # float32 holds every 24-bit sample exactly
+
+
+def dump_index(n, wl):
+    """The packets whose PCM --dump-outputs writes: a fixed seeded sample of the batch's n packets that fits DUMP_BYTES
+    next to the per-packet arrays, plus the first packet and the last (the short one)."""
+    per_packet = wl['cfg'].frame_length * wl['channels'] * np.dtype(dump_dtype(wl['bits'])).itemsize + 8
+    k = min(n, max(1, (DUMP_BYTES - 16 * n) // per_packet))
+    idx = np.random.default_rng(0).choice(n, size=k, replace=False)
+    return np.union1d(idx, [0, n - 1]).astype(np.int64)
+
+
+def write_dump(path, wl, idx, rows, out_bytes, status):
+    """rows: u8 [len(idx), >= frame_bytes], the PCM the timed path returned for packets idx; out_bytes, status: [n] of
+    every packet. Writes the arrays described in the module docstring."""
+    import oracle_lib as ol
+    ch, fl, bps = wl['channels'], wl['cfg'].frame_length, wl['cfg'].bps()
+    rows = np.ascontiguousarray(rows[:, :fl * ch * bps])
+    pcm = ol.pcm_bytes_to_int(rows.tobytes(), wl['bits'], ch).reshape(len(idx), fl * ch)
+    valid = np.where(status[idx] == 0, out_bytes[idx], 0).astype(np.int64) // bps
+    pcm[np.arange(fl * ch)[None, :] >= valid[:, None]] = 0  # bytes past out_bytes are not part of the result
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, 'pcm.npy'), pcm.reshape(len(idx), fl, ch).astype(dump_dtype(wl['bits'])))
+    np.save(os.path.join(path, 'pcm_packets.npy'), idx.astype(np.float64))
+    np.save(os.path.join(path, 'out_bytes.npy'), np.asarray(out_bytes).astype(np.float64))
+    np.save(os.path.join(path, 'status.npy'), np.asarray(status).astype(np.float64))
+
 
 class Pinned:
     """A pinned host array from the product's allocator."""
@@ -342,6 +387,14 @@ class Runner:
         prof = self.dec.get_profile()
         self.dec.set_profiling(False)
         return e0.elapsed_time(e1), prof.ms_decode / max(1, prof.launches_decode), int(prof.launches_decode)
+
+    def device_results(self, idx):
+        """What the last device step returned: (PCM rows of this shard's packets idx, out_bytes and status of all)."""
+        torch = self.torch
+        torch.cuda.synchronize()
+        sel = torch.from_numpy(np.ascontiguousarray(idx, dtype=np.int64)).cuda()
+        rows = self.d_pcm.view(max(1, self.n), self.stride)[sel, :self.dec.frame_bytes].cpu().numpy()
+        return rows, self.d_nb[:self.n].cpu().numpy().view(np.uint32), self.d_st[:self.n].cpu().numpy()
 
     def prepare_host(self):
         self.h_in = Pinned(self.pkg, len(self.host_bytes))
@@ -495,18 +548,17 @@ def library_record(pkg, torch, dev, rank, cores, steps, peak, dist, with_cpu):
 
 def api_legs(pkg, wl_c2, wl_c1, steps):
     """The drop-in API as a caller sees it, through the compiled C++ mirror (tools/api_bench.cpp)."""
-    import tempfile
     from m4a_writer import build_m4a
-    exe = os.path.join(ROOT, 'tools', 'build', 'api_bench')
+    exe = os.path.join(ROOT, 'tools', 'build', 'api_bench')  # built by build()
     src = os.path.join(ROOT, 'tools', 'api_bench.cpp')
     lib_dir = os.path.dirname(pkg.LIB_PATH)
-    os.makedirs(os.path.dirname(exe), exist_ok=True)
     hdr = os.path.join(ROOT, 'saprobe-alac_b200', 'host', 'alac.hpp')
-    if not os.path.exists(exe) or os.path.getmtime(exe) < max(os.path.getmtime(src), os.path.getmtime(hdr), os.path.getmtime(pkg.LIB_PATH)):
-        subprocess.run(['g++', '-std=c++17', '-O2', '-o', exe, src, '-L' + lib_dir, '-lalacb200', '-Wl,-rpath,' + lib_dir], check=True)
     out = {}
     with tempfile.TemporaryDirectory() as d:
         f = lambda n: os.path.join(d, n)
+        if not os.path.exists(exe) or os.path.getmtime(exe) < max(os.path.getmtime(src), os.path.getmtime(hdr), os.path.getmtime(pkg.LIB_PATH)):
+            exe = f('api_bench')  # missing or stale: compile a private copy, the tree may be read-only
+            subprocess.run(['g++', '-std=c++17', '-O2', '-o', exe, src, '-L' + lib_dir, '-lalacb200', '-Wl,-rpath,' + lib_dir], check=True)
         open(f('cookie'), 'wb').write(wl_c2['cookie'])
         wl_c2['packed'].tofile(f('packed'))
         wl_c2['offsets'].astype(np.uint64).tofile(f('offs'))
@@ -555,7 +607,10 @@ def main():
     ap.add_argument('--workload', default='c3', choices=sorted(WORKLOADS))
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--only-main', action='store_true', help='skip the sub-records (other configs, library batch, API legs)')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write what the timed path returned in its last step as DIR/*.npy')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     if args.warmup < 3 and args.impl == 'ours':
         args.warmup = 3
 
@@ -581,8 +636,11 @@ def main():
         out[:] = 1
         t0 = time.perf_counter()
         for _ in range(args.steps):
-            ol.decode_batch(wl['cfg'], wl['packed'], wl['offsets'], wl['sizes'], nthreads=cores, out=out)
+            _, nb, st = ol.decode_batch(wl['cfg'], wl['packed'], wl['offsets'], wl['sizes'], nthreads=cores, out=out)
         dt = time.perf_counter() - t0
+        if args.dump_outputs:
+            idx = dump_index(n, wl)
+            write_dump(args.dump_outputs, wl, idx, out[idx], nb, st)
         value = wl['frames'] * wl['channels'] * args.steps / dt
         line = {'impl': 'reference', 'metric': 'decoded PCM samples/s', 'value': value, 'unit': 'samples/s',
                 'n_gpus': args.gpus, 'steps': args.steps, 'warmup': args.warmup, 'ms_per_step': dt / args.steps * 1e3,
@@ -633,6 +691,15 @@ def main():
     e2e_s = run.time_host(e2e_steps, barrier)
     clocks = sampler.stop()
     barrier()
+    if args.dump_outputs:  # the host leg writes its own buffers: the device buffers still hold the last timed step
+        idx = dump_index(len(wl['sizes']), wl)
+        parts = [run.device_results(idx[(idx >= lo) & (idx < hi)] - lo)]
+        if dist is not None:
+            mine, parts = parts[0], [None] * world
+            dist.all_gather_object(parts, mine)  # contiguous shards in rank order: concatenation is batch order
+        if rank == 0:
+            write_dump(args.dump_outputs, wl, idx, *(np.concatenate([p[j] for p in parts]) for j in range(3)))
+        barrier()
 
     # ---- max over ranks of the times, sums of the work -------------------------------------------------------------
     t = torch.tensor([ms_total, e2e_s * 1e3, dec_ms], dtype=torch.float64, device='cuda')

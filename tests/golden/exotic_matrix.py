@@ -15,13 +15,19 @@ wrap at chanBits and the FIR sum can leave int32, where FFmpeg's arithmetic and 
 whose sample width exceeds 32 bits (32-bit pairs without shifted bytes, 32-bit escape pairs: "bps 33 is not
 implemented"), DSE / FIL elements and packets without an END tag (FFmpeg refuses them): build() returns None for a case
 FFmpeg rejects.
+
+The names of the cases FFmpeg confirmed are committed (exotic_confirmed.json, `python tests/golden/exotic_matrix.py`
+rewrites it), so that checked_cases() still yields those streams -- all of them from the test-side encoder and seeds --
+where the FFmpeg libraries are not installed.
 """
+import json
 import os
 import sys
 
 import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
+CONFIRMED_PATH = os.path.join(HERE, 'exotic_confirmed.json')
 sys.path.insert(0, os.path.dirname(HERE))
 import oracle_lib as ol  # noqa: E402
 from signals import make_signal  # noqa: E402
@@ -75,20 +81,30 @@ def ffmpeg_available():
         return False
 
 
-def build(case):
-    """-> (oracle config, [packets], source int64 [frames, ch]) after FFmpeg's decoder has returned the source for these
-    packets, or None when FFmpeg rejects the stream (sample width above 32 bits)."""
-    sys.path.insert(0, HERE)
-    import ffmpeg_alac as ff
+def encode(case):
+    """-> (oracle config, [packets], source int64 [frames, ch]) from the test-side encoder, or None when it has no
+    representation for a frame (a 32-bit pair that needs an escape element)."""
     rate = 48000
     x = make_signal(case['kind'], case['channels'], case['frames'], case['bits'], rate, seed=case['seed'])
     cfg = ol.Config.make(bit_depth=case['bits'], num_channels=case['channels'], sample_rate=rate, frame_length=case.get('frame_length', 4096))
     extra = {k: case[k] for k in ('pb_factor', 'den_shift', 'mix_bits', 'mix_res', 'force_escape', 'lfe_tag3', 'always_partial') if k in case}
     opts = ol.PacketOpts.make(min_order=case['orders'][0], max_order=case['orders'][1], bytes_shifted=case['shift'], mode=case['mode'], **extra)
     try:
-        packets = ol.encode_stream(cfg, x, opts)
-    except ValueError:  # the test-side encoder has no representation for this frame (32-bit pair that needs an escape element)
+        return cfg, ol.encode_stream(cfg, x, opts), x
+    except ValueError:
         return None
+
+
+def build(case):
+    """-> (oracle config, [packets], source int64 [frames, ch]) after FFmpeg's decoder has returned the source for these
+    packets, or None when FFmpeg rejects the stream (sample width above 32 bits)."""
+    sys.path.insert(0, HERE)
+    import ffmpeg_alac as ff
+    built = encode(case)
+    if built is None:
+        return None
+    cfg, packets, x = built
+    rate = cfg.sample_rate
     try:
         y = ff.alac_decode(ol.make_cookie(cfg, wrappers=1), packets, case['bits'], case['channels'], rate).T
     except (RuntimeError, ValueError):  # send_packet refused, or no frame came out
@@ -97,3 +113,24 @@ def build(case):
         return None
     assert np.array_equal(y, x), f"FFmpeg's decoder does not return the source for {case['name']}"
     return cfg, packets, x
+
+
+def checked_cases():
+    """-> [(case, cfg, packets, source)] of the streams FFmpeg's decoder returns the source for: confirmed now when the
+    FFmpeg libraries are present, else the committed list of confirmed cases."""
+    if ffmpeg_available():
+        built = ((case, build(case)) for case in exotic_cases())
+    else:
+        with open(CONFIRMED_PATH) as f:
+            names = set(json.load(f)['cases'])
+        built = ((case, encode(case)) for case in exotic_cases() if case['name'] in names)
+    return [(case, *b) for case, b in built if b is not None]
+
+
+if __name__ == '__main__':
+    assert ffmpeg_available(), 'confirming the cases needs the FFmpeg libraries'
+    names = [case['name'] for case, _, _, _ in checked_cases()]
+    with open(CONFIRMED_PATH, 'w') as f:
+        json.dump(dict(what="exotic_matrix cases whose packets FFmpeg's ALAC decoder (libavcodec 62.11.100) decodes to the source",
+                       cases=names), f, indent=0)
+    print(len(names), 'cases confirmed')
