@@ -147,14 +147,11 @@ __device__ __forceinline__ void mbar_arrive(uint64_t *bar) {
 // takes ~8000 cycles to produce, a whole stream ~1 M): mbarrier.try_wait with a suspend-time hint parks the warp in
 // hardware until the phase completes or the hint expires, so the poll loop issues a handful of instructions per wait
 // instead of one poll every ~20 cycles (__nanosleep returned almost at once in the round-1 captures: 90 M polls on c2).
-#ifndef ALACB200_WAIT
-#define ALACB200_WAIT 1
-#endif
-__device__ __forceinline__ void mbar_wait(uint64_t *bar, uint32_t parity, uint32_t backoff_ns = 0) {
+// `long_wait`: a warp that waits for a whole ring slot to be produced may stay suspended longer per try.
+__device__ __forceinline__ void mbar_wait(uint64_t *bar, uint32_t parity, bool long_wait = false) {
     const uint32_t addr = smem_u32(bar);
+    const uint32_t hint = long_wait ? 100000u : 2000u;  // ns the hardware may keep the warp suspended per try
     uint32_t done;
-#if ALACB200_WAIT == 1
-    const uint32_t hint = backoff_ns ? 100000u : 2000u;  // ns the hardware may keep the warp suspended per try
     for (;;) {
         asm volatile(
             "{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2, %3;\n\tselp.u32 %0, 1, 0, p;\n\t}"
@@ -163,50 +160,7 @@ __device__ __forceinline__ void mbar_wait(uint64_t *bar, uint32_t parity, uint32
             : "memory");
         if (done) break;
     }
-#else
-    uint32_t ns = backoff_ns;
-    for (;;) {
-        asm volatile(
-            "{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-            : "=r"(done)
-            : "r"(addr), "r"(parity)
-            : "memory");
-        if (done) break;
-        if (backoff_ns) {
-            __nanosleep(ns);
-#if ALACB200_WAIT == 2
-            ns = min(ns * 2u, 8000u);  // exponential back-off
-#endif
-        }
-    }
-#endif
 }
-
-// ---- hand-over between the two role warps ------------------------------------------------------------------------
-//   full[slot]   entropy -> predictor: the ring slot holds 32 codes per lane
-//   empty[slot]  predictor -> entropy: the slot may be refilled
-// mbarriers in shared memory (default). A waiting warp polls -- try_wait comes back within ~10 cycles whatever suspend
-// hint or nanosleep it is given -- but the polls are free: the same protocol on hardware named barriers (bar.arrive /
-// bar.sync, -DALACB200_NAMED_BARRIERS), where a waiting warp issues nothing at all, was bit-identical and 0.5-1.5 %
-// SLOWER when measured on the four-warp form of this kernel (profiles/r02a). The issue slots were never the limit; the
-// dependent chains of the role warps are.
-#ifdef ALACB200_NAMED_BARRIERS
-// barrier numbers as immediates, so that ptxas reserves the barriers the kernel uses (1..4; 0 is __syncthreads)
-#define ALACB200_BAR_CASES(OP)                                                                                              \
-    switch (id) {                                                                                                          \
-    case 1: asm volatile(OP " 1, 64;" ::: "memory"); break;                                                                \
-    case 2: asm volatile(OP " 2, 64;" ::: "memory"); break;                                                                \
-    case 3: asm volatile(OP " 3, 64;" ::: "memory"); break;                                                                \
-    default: asm volatile(OP " 4, 64;" ::: "memory"); break;                                                               \
-    }
-__device__ __forceinline__ void nbar_sync(uint32_t id) { ALACB200_BAR_CASES("bar.sync") }
-__device__ __forceinline__ void nbar_arrive(uint32_t id) { ALACB200_BAR_CASES("bar.arrive") }
-#endif
-struct DecShared;
-__device__ __forceinline__ void wait_full(DecShared &sm, uint32_t seq);
-__device__ __forceinline__ void arrive_full(DecShared &sm, uint32_t seq);
-__device__ __forceinline__ void wait_empty(DecShared &sm, uint32_t seq);
-__device__ __forceinline__ void arrive_empty(DecShared &sm, uint32_t seq);
 
 __device__ unsigned int g_sm_ticket[256];        // per-SM CTA counter (monotonic; only its value mod 4 is used)
 __device__ unsigned int g_sm_entropy_load[256];  // per SM: four 8-bit counts of resident entropy warps, by sub-partition
@@ -291,37 +245,22 @@ static_assert(offsetof(DecShared, fifo) == 0 && (FIFO_CHUNKS & (FIFO_CHUNKS - 1)
 static_assert(offsetof(DecShared, ring) % 16 == 0 && offsetof(DecShared, live_shift) % 16 == 0 && offsetof(DecShared, full_bar) % 8 == 0, "alignment");
 static_assert(sizeof(DecShared) + 1024 <= (228 * 1024) / CTAS_PER_SM, "eight CTAs per SM");
 
+// ---- hand-over between the two role warps ------------------------------------------------------------------------
+//   full[slot]   entropy -> predictor: the ring slot holds 32 codes per lane
+//   empty[slot]  predictor -> entropy: the slot may be refilled
+// mbarriers in shared memory. A waiting warp polls -- try_wait comes back within ~10 cycles whatever suspend hint or
+// nanosleep it is given -- but the polls are free: the same protocol on hardware named barriers (bar.arrive / bar.sync),
+// where a waiting warp issues nothing at all, was bit-identical and 0.5-1.5 % SLOWER when measured on the four-warp form
+// of this kernel (profiles/r02a). The issue slots were never the limit; the dependent chains of the role warps are.
+// Every lane arrives (32 arrivals per hand-over). One arrival by one lane after a __syncwarp() was bit-identical and
+// measured at +-0.4 % on every workload: the waiter's polls (a tenth of the instructions the kernel issues) are not caused
+// by the per-lane arrivals and cost nothing anybody else wanted.
 // `seq` is the ring sequence number of the slot (slot = seq % RING_SLOTS, phase = seq / RING_SLOTS)
-#ifdef ALACB200_NAMED_BARRIERS
-__device__ __forceinline__ void wait_full(DecShared &, uint32_t seq) { nbar_sync(1u + seq % RING_SLOTS); }
-__device__ __forceinline__ void arrive_full(DecShared &, uint32_t seq) { nbar_arrive(1u + seq % RING_SLOTS); }
-__device__ __forceinline__ void wait_empty(DecShared &, uint32_t seq) {  // the first RING_SLOTS uses find the ring empty
-    if (seq >= RING_SLOTS) nbar_sync(3u + seq % RING_SLOTS);
-}
-__device__ __forceinline__ void arrive_empty(DecShared &, uint32_t seq) { nbar_arrive(3u + seq % RING_SLOTS); }
-#else
-__device__ __forceinline__ void wait_full(DecShared &sm, uint32_t seq) { mbar_wait(&sm.full_bar[seq % RING_SLOTS], (seq / RING_SLOTS) & 1u, 200); }
-// Every lane arrives (32 arrivals per hand-over). One arrival by one lane after a __syncwarp() (-DALACB200_ARRIVE_ONE=1) is
-// bit-identical and was measured at +-0.4 % on every workload: the waiter's polls (a tenth of the instructions the kernel
-// issues) are not caused by the per-lane arrivals and cost nothing anybody else wanted.
-#ifndef ALACB200_ARRIVE_ONE
-#define ALACB200_ARRIVE_ONE 0
-#endif
-constexpr uint32_t BAR_ARRIVALS = ALACB200_ARRIVE_ONE ? 1u : 32u;
-__device__ __forceinline__ void warp_arrive(uint64_t *bar) {
-#if ALACB200_ARRIVE_ONE
-    __syncwarp();
-    uint32_t lane;
-    asm volatile("mov.u32 %0, %%laneid;" : "=r"(lane));
-    if (lane == 0) mbar_arrive(bar);
-#else
-    mbar_arrive(bar);
-#endif
-}
-__device__ __forceinline__ void arrive_full(DecShared &sm, uint32_t seq) { warp_arrive(&sm.full_bar[seq % RING_SLOTS]); }
+constexpr uint32_t BAR_ARRIVALS = 32u;
+__device__ __forceinline__ void wait_full(DecShared &sm, uint32_t seq) { mbar_wait(&sm.full_bar[seq % RING_SLOTS], (seq / RING_SLOTS) & 1u, true); }
+__device__ __forceinline__ void arrive_full(DecShared &sm, uint32_t seq) { mbar_arrive(&sm.full_bar[seq % RING_SLOTS]); }
 __device__ __forceinline__ void wait_empty(DecShared &sm, uint32_t seq) { mbar_wait(&sm.empty_bar[seq % RING_SLOTS], ((seq / RING_SLOTS) & 1u) ^ 1u); }
-__device__ __forceinline__ void arrive_empty(DecShared &sm, uint32_t seq) { warp_arrive(&sm.empty_bar[seq % RING_SLOTS]); }
-#endif
+__device__ __forceinline__ void arrive_empty(DecShared &sm, uint32_t seq) { mbar_arrive(&sm.empty_bar[seq % RING_SLOTS]); }
 
 // job meta word
 enum : uint32_t { JOB_INACTIVE = 0, JOB_REG = 1, JOB_GENERIC = 2, JOB_EXIT = 3 };  // JOB_EXIT: the group is finished
@@ -623,9 +562,6 @@ constexpr int E_UNROLL = ALACB200_EUNROLL;
 #define ALACB200_PUNROLL 2
 #endif
 constexpr int P_UNROLL = ALACB200_PUNROLL;
-#ifndef ALACB200_FIRSPLIT
-#define ALACB200_FIRSPLIT 1
-#endif
 #ifndef ALACB200_QUNROLL
 #define ALACB200_QUNROLL 2
 #endif
@@ -1108,6 +1044,79 @@ __device__ __forceinline__ uint32_t shift_field(const uint32_t *row_words, uint3
     return win >> (32u - sb);
 }
 
+// ---- the writer rules of stage 3 (WriteStereo*/WriteMono*, matrix.go:30-301), one copy for every emit path -----------
+// One frame: un-mix (matrix.go:40-41), 20-bit samples moved up by 4, then the shift buffer merge (matrix.go:132-135,
+// :270-272: BitBuffer.Read of sb bits at bit `rel` of the staged shift row). A mono frame leaves `right` alone.
+__device__ __forceinline__ void writer_frame(int32_t &left, int32_t &right, bool stereo, int32_t mix_res, uint32_t mix_bits,
+                                             bool depth20, uint32_t sb, const uint32_t *shift_row, uint32_t rel) {
+    if (stereo && mix_res != 0) {
+        const int32_t v = right;
+        left = left + v - sar_go(mix_res * v, mix_bits);
+        right = left - v;
+    }
+    if (depth20) {
+        left = (int32_t)((uint32_t)left << 4);
+        right = (int32_t)((uint32_t)right << 4);
+    }
+    if (sb) {
+        left = (int32_t)shl_go((uint32_t)left, sb) | (int32_t)shift_field(shift_row, rel, sb);
+        if (stereo) right = (int32_t)shl_go((uint32_t)right, sb) | (int32_t)shift_field(shift_row, rel + sb, sb);
+    }
+}
+
+// OR frame q of a batch -- the BPS little-endian bytes of `left`, then, for WIDTH 2, those of `right` -- into the packed
+// words ow[] of the batch; a frame that is not kept (past the sample count, decoder.go:120, :127) stays zero.
+template <int BPS, int WIDTH>
+__device__ __forceinline__ void pack_frame(uint32_t *ow, int q, int32_t left, int32_t right, bool keep) {
+    constexpr int FB = BPS * WIDTH;
+    constexpr uint64_t lmask = BPS == 4 ? 0xffffffffull : ((1ull << (8 * BPS)) - 1ull);
+    uint64_t v = (uint64_t)(uint32_t)left & lmask;
+    if (WIDTH == 2) v |= ((uint64_t)(uint32_t)right & lmask) << (8 * BPS);
+    if (!keep) v = 0;
+    const int bit = q * FB * 8;  // static after unrolling
+    const int wi = bit / 32, sh = bit % 32;
+    ow[wi] |= (uint32_t)(v << sh);
+    if (sh + FB * 8 > 32) ow[wi + 1] |= (uint32_t)(v >> (32 - sh));
+    if (sh + FB * 8 > 64) ow[wi + 2] |= (uint32_t)(v >> (64 - sh));
+}
+
+// Store the packed words of FRAMES frames (NW4 x 16 bytes) from frame f0 on to a packet slot: 128-bit stores when the
+// batch is whole and the slot 16-byte aligned, else 32-bit stores and the bytes of a last partial word (the last, short
+// batch of a frame length that is not a multiple of FRAMES; 24-bit pairs are a multiple of 4 bytes only for an even
+// number of frames).
+template <int NW4, int FRAMES>
+__device__ __forceinline__ void store_words(uint8_t *slot, uint32_t f0, uint32_t frame_bytes, uint32_t frame_length,
+                                            bool vec_ok, const uint32_t *ow) {
+    uint8_t *dst = slot + (size_t)f0 * frame_bytes;
+    const uint32_t frames_here = min((uint32_t)FRAMES, frame_length - f0);
+    if (frames_here == (uint32_t)FRAMES && vec_ok) {
+#pragma unroll
+        for (int k = 0; k < NW4; k++)
+            reinterpret_cast<uint4 *>(dst)[k] = make_uint4(ow[4 * k], ow[4 * k + 1], ow[4 * k + 2], ow[4 * k + 3]);
+    } else {
+        const uint32_t nb = frames_here * frame_bytes;
+#pragma unroll
+        for (int k = 0; k < 4 * NW4; k++) {
+            if ((uint32_t)(4 * k + 4) <= nb) reinterpret_cast<uint32_t *>(dst)[k] = ow[k];
+            else
+                for (int j = 0; j < 4; j++)
+                    if ((uint32_t)(4 * k + j) < nb) dst[4 * k + j] = (uint8_t)(ow[k] >> (8 * j));
+        }
+    }
+}
+
+// Word k of a shift row staged from packet byte rel_pk on (gsrc: the row's 4-byte aligned global address): one aligned
+// load, or, where the word runs past the packet end, its bytes one by one with those outside the packet read as zero
+// (bitbuffer.go:36-51).
+__device__ __forceinline__ uint32_t shift_word(const Packet &pk, int64_t rel_pk, uint32_t k, const uint32_t *gsrc) {
+    const int64_t b_first = rel_pk + 4 * (int64_t)k;
+    if (b_first + 4 <= (int64_t)pk.size) return __ldg(gsrc + k);
+    uint32_t w = 0;
+    for (int j = 0; j < 4; j++)
+        if (b_first + j >= 0 && b_first + j < (int64_t)pk.size) w |= (uint32_t)__ldg(pk.p + (b_first + j)) << (8 * j);
+    return w;
+}
+
 // What the predictor warp needs to emit PCM itself (2-channel streams), apart from the per-lane words in
 // DecShared::live_ctx: launch facts that rematerialise from the kernel's parameter bank. Only ever handed to inlined
 // code, so it never has an address.
@@ -1209,47 +1218,10 @@ __device__ __noinline__ void live_emit_generic(DecShared &sm, uint32_t lane, con
         for (int q = 0; q < EB; q++) {
             const uint32_t jq = half * EB + (uint32_t)q;
             int32_t left = sm.live_u[jq][lane], right = vsrc[jq * 32u];
-            if (mix_res != 0) {  // matrix.go:40-41
-                const int32_t v = right;
-                left = left + v - sar_go(mix_res * v, mix_bits);
-                right = left - v;
-            }
-            if (depth20) {
-                left = (int32_t)((uint32_t)left << 4);
-                right = (int32_t)((uint32_t)right << 4);
-            }
-            if (sb) {  // shift buffer merge, matrix.go:132-135
-                const uint32_t rel = rel0 + jq * 2u * sb;
-                left = (int32_t)shl_go((uint32_t)left, sb) | (int32_t)shift_field(shrow, rel, sb);
-                right = (int32_t)shl_go((uint32_t)right, sb) | (int32_t)shift_field(shrow, rel + sb, sb);
-            }
-            constexpr uint64_t lmask = BPS == 4 ? 0xffffffffull : ((1ull << (8 * BPS)) - 1ull);
-            uint64_t v = ((uint64_t)(uint32_t)left & lmask) | (((uint64_t)(uint32_t)right & lmask) << (8 * BPS));
-            if ((uint32_t)q >= cnt) v = 0;  // frames past the sample count stay zero (decoder.go:120, :127)
-            const int bit = q * FB * 8;
-            const int wi = bit / 32, sh = bit % 32;
-            ow[wi] |= (uint32_t)(v << sh);
-            if (sh + FB * 8 > 32) ow[wi + 1] |= (uint32_t)(v >> (32 - sh));
-            if (sh + FB * 8 > 64) ow[wi + 2] |= (uint32_t)(v >> (64 - sh));
+            writer_frame(left, right, true, mix_res, mix_bits, depth20, sb, shrow, rel0 + jq * 2u * sb);
+            pack_frame<BPS, 2>(ow, q, left, right, (uint32_t)q < cnt);
         }
-        if (live_lane) {
-            uint8_t *dst = lc.slot + (size_t)f0 * FB;
-            const uint32_t frames_here = min((uint32_t)EB, lc.frame_length - f0);
-            if (frames_here == EB && lc.vec_ok) {
-#pragma unroll
-                for (int k = 0; k < FB; k++)
-                    reinterpret_cast<uint4 *>(dst)[k] = make_uint4(ow[4 * k], ow[4 * k + 1], ow[4 * k + 2], ow[4 * k + 3]);
-            } else {
-                const uint32_t nb = frames_here * FB;  // 24-bit pairs: a multiple of 4 only for an even number of frames
-#pragma unroll
-                for (int k = 0; k < 4 * FB; k++) {
-                    if ((uint32_t)(4 * k + 4) <= nb) reinterpret_cast<uint32_t *>(dst)[k] = ow[k];
-                    else
-                        for (int j = 0; j < 4; j++)
-                            if ((uint32_t)(4 * k + j) < nb) dst[4 * k + j] = (uint8_t)(ow[k] >> (8 * j));
-                }
-            }
-        }
+        if (live_lane) store_words<FB, EB>(lc.slot, f0, FB, lc.frame_length, lc.vec_ok, ow);
     }
 }
 
@@ -1258,28 +1230,6 @@ __device__ __forceinline__ void unmix(int32_t u, int32_t v, int32_t mix_res, uin
     const int32_t l = u + v - sar_go(mix_res * v, mix_bits);
     left = mix_res != 0 ? l : u;
     right = mix_res != 0 ? l - v : v;
-}
-
-// Store the packed words of FRAMES frames (NW4 x 16 bytes) to the lane's packet slot.
-template <int NW4, int FRAMES>
-__device__ __forceinline__ void store_batch(const LiveOut &lc, uint32_t f0, uint32_t fb, const uint32_t *ow, bool live_lane) {
-    if (!live_lane) return;
-    uint8_t *dst = lc.slot + (size_t)f0 * fb;
-    const uint32_t frames_here = min((uint32_t)FRAMES, lc.frame_length - f0);
-    if (frames_here == (uint32_t)FRAMES && lc.vec_ok) {
-#pragma unroll
-        for (int k = 0; k < NW4; k++)
-            reinterpret_cast<uint4 *>(dst)[k] = make_uint4(ow[4 * k], ow[4 * k + 1], ow[4 * k + 2], ow[4 * k + 3]);
-    } else {
-        const uint32_t nb = frames_here * fb;  // 24-bit pairs: a multiple of 4 only for an even number of frames
-#pragma unroll
-        for (int k = 0; k < 4 * NW4; k++) {
-            if ((uint32_t)(4 * k + 4) <= nb) reinterpret_cast<uint32_t *>(dst)[k] = ow[k];
-            else
-                for (int j = 0; j < 4; j++)
-                    if ((uint32_t)(4 * k + j) < nb) dst[4 * k + j] = (uint8_t)(ow[k] >> (8 * j));
-        }
-    }
 }
 
 // Emit the 32 frames of chunk `ck` of a live pair: V from the ring slot, U from live_u, shift bytes from live_shift; four
@@ -1335,7 +1285,7 @@ __device__ __forceinline__ void live_emit(DecShared &sm, uint32_t lane, const Li
                 ow[3 * pr + 1] = __byte_perm(x24[1], x24[2], 0x5421);  // R0 R0 L1 L1
                 ow[3 * pr + 2] = __byte_perm(x24[2], x24[3], 0x6542);  // L1 R1 R1 R1
             }
-            store_batch<3, 8>(lc, f0, 6u, ow, live_lane);
+            if (live_lane) store_words<3, 8>(lc.slot, f0, 6u, lc.frame_length, lc.vec_ok, ow);
         } else {
             uint32_t ow[8];
 #pragma unroll
@@ -1347,7 +1297,7 @@ __device__ __forceinline__ void live_emit(DecShared &sm, uint32_t lane, const Li
                 if ((uint32_t)q >= cnt) w = 0;
                 ow[q] = w;
             }
-            store_batch<2, 8>(lc, f0, 4u, ow, live_lane);
+            if (live_lane) store_words<2, 8>(lc.slot, f0, 4u, lc.frame_length, lc.vec_ok, ow);
         }
     }
 }
@@ -1432,11 +1382,7 @@ __device__ __forceinline__ void stream_reg(DecShared &sm, uint32_t lane, uint32_
     // steady-state body below runs instead of the general one: no warm-up arithmetic, and the early-exit ladder of
     // predictor.go:137-185 in a sign-folded form -- with E = del0 for a positive residual and ~del0 for a negative one,
     // both ladders are "E -= weight * q; go on while E >= thr", q = |diff| >> denShift rounded down / up, thr = 1 / 0.
-#ifdef ALACB200_NO_STEADY
-    const bool steady_ok = false;
-#else
     const bool steady_ok = !MODE && __all_sync(FULL_MASK, !active || (fir_order && jb.chan_bits <= 31u));
-#endif
     const uint32_t den_mask = (1u << den) - 1u;
     // One ring slot = wait for it, start the fetches its emission needs, run a sample loop over it, emit or park it, hand
     // it back. Two loops over the slots instead of one with both bodies in it: the general body takes the first slot of
@@ -1546,22 +1492,15 @@ __device__ __forceinline__ void stream_reg(DecShared &sm, uint32_t lane, uint32_
                 else top = sel4 ? h[4] : sel5 ? h[5] : h[6];
                 int32_t d[T];
                 int32_t sum = den_half;
-#if ALACB200_FIRSPLIT
                 int32_t sum_b = 0;  // two accumulators: the dependent IMAD chain of the FIR is half as long (wrap-around sums commute)
-#endif
 #pragma unroll
                 for (int t = 0; t < T; t++) {
                     d[t] = top - h[t];
                     if (t >= 4) d[t] &= (int32_t)tmask[t];  // orders start at 4: taps 0..3 always live
-#if ALACB200_FIRSPLIT
                     if (t & 1) sum_b -= c[t] * d[t];
-                    else
-#endif
-                    sum -= c[t] * d[t];
+                    else sum -= c[t] * d[t];
                 }
-#if ALACB200_FIRSPLIT
                 sum += sum_b;
-#endif
                 const int32_t x = sext_bits(r + top + (sum >> den), jb.chan_bits);
                 const int32_t smask = r >> 31;                       // 0 / -1
                 const int32_t nsone = -(smask | 1);                  // -1 for r > 0, +1 for r < 0: coef -= sign(diff) * sign(r)
@@ -1867,20 +1806,8 @@ __device__ __forceinline__ void emit_frames(const EmitOp &o, uint8_t *row, const
             const int32_t i = ib + q;
             if (i < o.i_hi) {
                 int32_t left = lu[q], right = o.stereo ? lv[q] : 0;
-                if (o.stereo && o.mix_res != 0) {  // matrix.go:40-41
-                    const int32_t v = right;
-                    left = left + v - sar_go(o.mix_res * v, o.mix_bits);
-                    right = left - v;
-                }
-                if (o.depth20) {
-                    left = (int32_t)((uint32_t)left << 4);
-                    right = (int32_t)((uint32_t)right << 4);
-                }
-                if (o.sb) {  // shift buffer merge, matrix.go:132-135, :270-272 (BitBuffer.Read of sb bits)
-                    const uint32_t rel = o.rel0 + (uint32_t)(i - o.i_lo) * o.width * o.sb;
-                    left = (int32_t)shl_go((uint32_t)left, o.sb) | (int32_t)shift_field(shrow_words, rel, o.sb);
-                    if (o.stereo) right = (int32_t)shl_go((uint32_t)right, o.sb) | (int32_t)shift_field(shrow_words, rel + o.sb, o.sb);
-                }
+                writer_frame(left, right, o.stereo, o.mix_res, o.mix_bits, o.depth20, o.sb, shrow_words,
+                             o.rel0 + (uint32_t)(i - o.i_lo) * o.width * o.sb);
                 tile_store<BPS>(row + (uint32_t)(i - o.s0) * o.fb + o.out_off, left, right, o.stereo);
             }
         }
@@ -1941,18 +1868,7 @@ __device__ __forceinline__ void emit_direct(const EmitArgs &x, const DevConfig &
             const uint32_t *gsrc = reinterpret_cast<const uint32_t *>(ga);
             uint32_t wbuf[SROW - 2];
 #pragma unroll
-            for (uint32_t k = 0; k < SROW - 2; k++) {
-                const int64_t b_first = rel_pk + 4 * (int64_t)k;
-                uint32_t w = 0;
-                if (k < nw) {
-                    if (b_first + 4 <= (int64_t)pk.size) w = __ldg(gsrc + k);
-                    else {  // bytes at or past the packet end read as zero (bitbuffer.go:36-51)
-                        for (int j = 0; j < 4; j++)
-                            if (b_first + j >= 0 && b_first + j < (int64_t)pk.size) w |= (uint32_t)__ldg(pk.p + (b_first + j)) << (8 * j);
-                    }
-                }
-                wbuf[k] = w;
-            }
+            for (uint32_t k = 0; k < SROW - 2; k++) wbuf[k] = k < nw ? shift_word(pk, rel_pk, k, gsrc) : 0u;
 #pragma unroll
             for (uint32_t k = 0; k < SROW - 2; k++) myrow[k] = wbuf[k];
             myrow[SROW - 2] = 0;
@@ -1966,49 +1882,12 @@ __device__ __forceinline__ void emit_direct(const EmitArgs &x, const DevConfig &
 #pragma unroll
         for (int q = 0; q < EB; q++) {
             int32_t left = lu[q], right = stereo ? lv[q] : 0;
-            if (stereo && mix_res != 0) {  // matrix.go:40-41
-                const int32_t v = right;
-                left = left + v - sar_go(mix_res * v, mix_bits);
-                right = left - v;
-            }
-            if (depth20) {
-                left = (int32_t)((uint32_t)left << 4);
-                right = (int32_t)((uint32_t)right << 4);
-            }
-            if (sb) {  // shift buffer merge, matrix.go:132-135, :270-272
-                const uint32_t rel = rel0 + (uint32_t)q * WIDTH * sb;
-                left = (int32_t)shl_go((uint32_t)left, sb) | (int32_t)shift_field(myrow, rel, sb);
-                if (stereo) right = (int32_t)shl_go((uint32_t)right, sb) | (int32_t)shift_field(myrow, rel + sb, sb);
-            }
-            constexpr uint64_t lmask = BPS == 4 ? 0xffffffffull : ((1ull << (8 * BPS)) - 1ull);
-            uint64_t v = (uint64_t)(uint32_t)left & lmask;
-            if (stereo) v |= ((uint64_t)(uint32_t)right & lmask) << (8 * BPS);
-            if ((uint32_t)q >= cnt) v = 0;  // frames past the sample count stay zero
-            const int bit = q * FB * 8;  // static after unrolling
-            const int wi = bit / 32, sh = bit % 32;
-            ow[wi] |= (uint32_t)(v << sh);
-            if (sh + FB * 8 > 32) ow[wi + 1] |= (uint32_t)(v >> (32 - sh));
-            if (sh + FB * 8 > 64) ow[wi + 2] |= (uint32_t)(v >> (64 - sh));
+            writer_frame(left, right, stereo, mix_res, mix_bits, depth20, sb, myrow, rel0 + (uint32_t)q * WIDTH * sb);
+            pack_frame<BPS, WIDTH>(ow, q, left, right, (uint32_t)q < cnt);
         }
         // ---- store: FB x 16 bytes to the lane's own packet slot ---------------------------------------------------
-        if (valid && f0 >= first_frame) {  // frames below first_frame were emitted live by the predictor warp
-            uint8_t *dst = slot + (size_t)f0 * FB;
-            const uint32_t frames_here = min((uint32_t)EB, cfg.frame_length - f0);
-            if (frames_here == EB && vec_ok) {
-#pragma unroll
-                for (int k = 0; k < FB; k++)
-                    reinterpret_cast<uint4 *>(dst)[k] = make_uint4(ow[4 * k], ow[4 * k + 1], ow[4 * k + 2], ow[4 * k + 3]);
-            } else {  // last, short batch of an odd frame length, or a slot that is only 4-byte aligned
-                const uint32_t nb = frames_here * FB;
-#pragma unroll
-                for (int k = 0; k < 4 * FB; k++) {
-                    if ((uint32_t)(4 * k + 4) <= nb) reinterpret_cast<uint32_t *>(dst)[k] = ow[k];
-                    else
-                        for (int j = 0; j < 4; j++)
-                            if ((uint32_t)(4 * k + j) < nb) dst[4 * k + j] = (uint8_t)(ow[k] >> (8 * j));
-                }
-            }
-        }
+        if (valid && f0 >= first_frame)  // frames below first_frame were emitted live by the predictor warp
+            store_words<FB, EB>(slot, f0, FB, cfg.frame_length, vec_ok, ow);
     }
 }
 
@@ -2084,15 +1963,9 @@ __device__ __forceinline__ void emit_rows(const EmitArgs &x, const DevConfig &cf
                             wbuf[4 * k] = v.x; wbuf[4 * k + 1] = v.y; wbuf[4 * k + 2] = v.z; wbuf[4 * k + 3] = v.w;
                         }
                     } else {
+                        const uint32_t *gsrc = reinterpret_cast<const uint32_t *>(ga);
 #pragma unroll 1
-                        for (uint32_t k = 0; k < SHIFT_WORDS; k++) {
-                            const int64_t b_first = rel_pk + 4 * (int64_t)k;
-                            uint32_t w = 0;
-                            if (k < nw)
-                                for (int j = 0; j < 4; j++)
-                                    if (b_first + j >= 0 && b_first + j < (int64_t)pk.size) w |= (uint32_t)__ldg(pk.p + (b_first + j)) << (8 * j);
-                            shrow[k] = w;
-                        }
+                        for (uint32_t k = 0; k < SHIFT_WORDS; k++) shrow[k] = k < nw ? shift_word(pk, rel_pk, k, gsrc) : 0u;
 #pragma unroll
                         for (uint32_t k = 0; k < SHIFT_WORDS; k++) wbuf[k] = shrow[k];
                     }
@@ -2108,20 +1981,7 @@ __device__ __forceinline__ void emit_rows(const EmitArgs &x, const DevConfig &cf
                 for (int q = 0; q < FR; q++) {
                     if ((uint32_t)q < cnt) {
                         int32_t left = lu[q], right = stereo ? lv[q] : 0;
-                        if (stereo && mix_res != 0) {  // matrix.go:40-41
-                            const int32_t v = right;
-                            left = left + v - sar_go(mix_res * v, mix_bits);
-                            right = left - v;
-                        }
-                        if (depth20) {
-                            left = (int32_t)((uint32_t)left << 4);
-                            right = (int32_t)((uint32_t)right << 4);
-                        }
-                        if (sb) {  // shift buffer merge, matrix.go:132-135, :270-272 (BitBuffer.Read of sb bits)
-                            const uint32_t rel = rel0 + (uint32_t)q * width * sb;
-                            left = (int32_t)shl_go((uint32_t)left, sb) | (int32_t)shift_field(shrow, rel, sb);
-                            if (stereo) right = (int32_t)shl_go((uint32_t)right, sb) | (int32_t)shift_field(shrow, rel + sb, sb);
-                        }
+                        writer_frame(left, right, stereo, mix_res, mix_bits, depth20, sb, shrow, rel0 + (uint32_t)q * width * sb);
                         tile_store<BPS>(dstb + (uint32_t)q * fb, left, right, stereo);
                     }
                 }
@@ -2265,16 +2125,9 @@ __host__ __device__ inline uint32_t emit_tile_frames(uint32_t frame_bytes, uint3
     return tl >= 16u ? (tl & ~15u) : (tl & ~3u);  // keep TL*fb a multiple of 16 where possible (128-bit stores)
 }
 
-#ifndef ALACB200_TAIL_INLINE
-#define ALACB200_TAIL_INLINE 1
-#endif
-#if ALACB200_TAIL_INLINE
-#define ALACB200_TAIL_FN __forceinline__
-#else
-#define ALACB200_TAIL_FN __noinline__
-#endif
+// Inlined into decode_cta: an out-of-line tail was measured and made no difference.
 template <int NWARPS>
-__device__ ALACB200_TAIL_FN void emit_group(const EmitArgs &x, const DevConfig &cfg, uint32_t group, uint8_t *smem,
+__device__ __forceinline__ void emit_group(const EmitArgs &x, const DevConfig &cfg, uint32_t group, uint8_t *smem,
                                            uint32_t smem_bytes) {
     const uint32_t lane = threadIdx.x & 31u, warp = threadIdx.x >> 5;
     const uint32_t fb = cfg.num_channels * cfg.bps;  // bytes per frame
@@ -2299,6 +2152,8 @@ __device__ ALACB200_TAIL_FN void emit_group(const EmitArgs &x, const DevConfig &
     const uint32_t max_ops = __reduce_max_sync(FULL_MASK, nops);
     // direct path when, for every packet of the group, one element covers the whole frame (or nothing is written)
     {
+        // cleared field by field, pad_ left out (it is only read when nops == 1): `OpDesc op0{}` makes ptxas spill more
+        // in both kernel builds
         OpDesc op0;
         op0.n = 0; op0.shift_bitpos = 0; op0.kind = 0; op0.out_chan = 0; op0.slot = 0; op0.shift = 0; op0.mix_bits = 0; op0.mix_res = 0;
         if (nops == 1) op0 = desc->ops[0];
@@ -2390,8 +2245,7 @@ __device__ ALACB200_TAIL_FN void emit_group(const EmitArgs &x, const DevConfig &
         __syncwarp();
 #pragma unroll 1
         for (uint32_t e = 0; e < max_ops; e++) {
-            OpDesc op;
-            op.n = 0; op.shift_bitpos = 0; op.kind = 0; op.out_chan = 0; op.slot = 0; op.shift = 0; op.mix_bits = 0; op.mix_res = 0;
+            OpDesc op{};
             if (e < nops) op = desc->ops[e];
             const bool stereo = op.kind == 2;
             const uint32_t sb = (merges_shift ? (uint32_t)op.shift : 0u) * 8u;
@@ -2415,16 +2269,7 @@ __device__ ALACB200_TAIL_FN void emit_group(const EmitArgs &x, const DevConfig &
                 uint32_t *myrow = shw + (size_t)lane * EMIT_SHIFT_ROW_WORDS;
                 const uint32_t *gsrc = reinterpret_cast<const uint32_t *>(ga);
 #pragma unroll 8
-                for (uint32_t k = 0; k < nw; k++) {
-                    const int64_t b_first = rel_pk + 4 * (int64_t)k;
-                    uint32_t w = 0;
-                    if (b_first + 4 <= (int64_t)pk.size) w = __ldg(gsrc + k);
-                    else {  // bytes at or past the packet end read as zero (bitbuffer.go:36-51)
-                        for (int j = 0; j < 4; j++)
-                            if (b_first + j >= 0 && b_first + j < (int64_t)pk.size) w |= (uint32_t)__ldg(pk.p + (b_first + j)) << (8 * j);
-                    }
-                    myrow[k] = w;
-                }
+                for (uint32_t k = 0; k < nw; k++) myrow[k] = shift_word(pk, rel_pk, k, gsrc);
                 myrow[nw] = 0;
                 myrow[nw + 1u] = 0;
                 rel0 = lead_bytes * 8u + (first_bit & 7u);
@@ -2442,26 +2287,12 @@ __device__ ALACB200_TAIL_FN void emit_group(const EmitArgs &x, const DevConfig &
                     else if (bps == 2) emit_frames<2>(eo, row, shrow_words);
                     else emit_frames<4>(eo, row, shrow_words);
                 } else {  // a pair spilling over the frame end (non-canonical element order): clip byte by byte
-                    const int32_t mix_res = op.mix_res;
-                    const uint32_t mix_bits = op.mix_bits;
+                    const uint32_t *shrow_words = shw + (size_t)lane * EMIT_SHIFT_ROW_WORDS;
 #pragma unroll 1
                     for (int32_t i = i_lo; i < i_hi; i++) {
                         int32_t left = su[(size_t)i * 32u], right = stereo ? sv[(size_t)i * 32u] : 0;
-                        if (stereo && mix_res != 0) {  // matrix.go:40-41
-                            const int32_t v = right;
-                            left = left + v - sar_go(mix_res * v, mix_bits);
-                            right = left - v;
-                        }
-                        if (depth20) {
-                            left = (int32_t)((uint32_t)left << 4);
-                            right = (int32_t)((uint32_t)right << 4);
-                        }
-                        if (sb) {
-                            const uint32_t rel = rel0 + (uint32_t)(i - i_lo) * width * sb;
-                            const uint32_t *shrow_words = shw + (size_t)lane * EMIT_SHIFT_ROW_WORDS;
-                            left = (int32_t)shl_go((uint32_t)left, sb) | (int32_t)shift_field(shrow_words, rel, sb);
-                            if (stereo) right = (int32_t)shl_go((uint32_t)right, sb) | (int32_t)shift_field(shrow_words, rel + sb, sb);
-                        }
+                        writer_frame(left, right, stereo, op.mix_res, op.mix_bits, depth20, sb, shrow_words,
+                                     rel0 + (uint32_t)(i - i_lo) * width * sb);
                         const int32_t off = i * (int32_t)fb + (int32_t)op.out_chan * bps;
                         tile_put(row, lo_byte, hi_byte, off, left, bps);
                         if (stereo) tile_put(row, lo_byte, hi_byte, off + bps, right, bps);
@@ -2518,12 +2349,10 @@ __device__ __forceinline__ void decode_cta(
     asm volatile("mov.u32 %0, %%smid;" : "=r"(smid));
     asm volatile("mov.u32 %0, %%warpid;" : "=r"(hw_warp));
     if (threadIdx.x == 0) {
-#ifndef ALACB200_NAMED_BARRIERS
         for (int s = 0; s < RING_SLOTS; s++) {
             mbar_init(&sm.full_bar[s], BAR_ARRIVALS);
             mbar_init(&sm.empty_bar[s], BAR_ARRIVALS);
         }
-#endif
         sm.group = atomicAdd(&counters[0], 1u);
     }
     if (lane == 0) sm.warp_smsp[warp] = hw_warp & 3u;  // %warpid is a hint, but any assignment of roles is correct
@@ -2599,11 +2428,7 @@ __device__ __forceinline__ void decode_cta(
         uint8_t *__restrict__ pcm_out, uint64_t out_stride, uint32_t *__restrict__ out_bytes,                              \
         int32_t *__restrict__ status, uint32_t *__restrict__ counters
 // The throughput build (big batches) ...
-#ifdef ALACB200_TP_MAXNREG
-__global__ void __maxnreg__(ALACB200_TP_MAXNREG) alac_decode_kernel(ALACB200_KERNEL_PARAMS) {
-#else
 __global__ void __launch_bounds__(DEC_THREADS, CTAS_PER_SM) alac_decode_kernel(ALACB200_KERNEL_PARAMS) {
-#endif
     decode_cta(packed, offsets, sizes, npackets, cfg, scratch, descs, pcm_out, out_stride, out_bytes, status, counters);
 }
 // ... and the register-rich build for batches of at most one wave of it.
