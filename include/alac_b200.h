@@ -140,6 +140,32 @@ int32_t alacb200_decode_packets_device(alacb200_decoder *dec, const uint8_t *d_p
                                        uint8_t *d_pcm_out, uint64_t out_stride, uint32_t *d_out_bytes,
                                        int32_t *d_status, void *stream);
 
+/* Channel-planar typed samples on DEVICE buffers (alacb200_decode_planar_device). Every type is defined on the container
+ * value, the sign-extended bps-byte little-endian sample of the interleaved PCM (a 20-bit sample is the stored value,
+ * i.e. << 4):
+ *   S16  int16, the container value; 16-bit streams only
+ *   S32  int32, the container value
+ *   F32  float, value * 2^-(8*bps-1), int-to-float rounded to nearest even: 16/20/24-bit values are exact and full
+ *        scale maps to [-1, 1) */
+enum { ALACB200_SAMPLES_S16 = 1, ALACB200_SAMPLES_S32 = 2, ALACB200_SAMPLES_F32 = 3 };
+
+/* DecodePackets on DEVICE buffers into channel-planar samples. Packet i's frames land in
+ * d_out[c*channel_stride + frame_start[i] .. frame_start[i+1]) of every channel c. A failed packet
+ * contributes no frames. d_frame_start has n+1 entries, and [n] is the total. channel_stride
+ * >= n*frame_length (elements). Frames between the total and channel_stride are not written.
+ * Same contract as alacb200_decode_packets_device for d_packed (16-byte aligned, readable for packed_bytes rounded
+ * up to 16, packets inside it), the stream and the decoder's scratch; d_status[n] gets the status words; d_out must
+ * be aligned to its element size. Enqueued on `stream` without synchronising: the decode kernel into an interleaved
+ * intermediate, the frame scan, the planar pass. The intermediate (n slots of max_packet_pcm_bytes rounded up to 16,
+ * plus n*4 bytes) comes from the device's stream-ordered pool and is freed on `stream` at the end of the call: it is at
+ * most the size of the output, and the decoder keeps no memory that grows with n between calls. n == 0 writes
+ * d_frame_start[0] = 0. ALACB200_E_ARG for an unknown sample_type, S16 on a stream that is not 16-bit, a NULL pointer
+ * (only d_frame_start when n == 0), channel_stride < n*frame_length, or a misaligned d_out or d_packed. */
+int32_t alacb200_decode_planar_device(alacb200_decoder *dec, const uint8_t *d_packed, uint64_t packed_bytes,
+                                      const uint64_t *d_offsets, const uint32_t *d_sizes, uint32_t n,
+                                      int32_t sample_type, void *d_out, uint64_t channel_stride,
+                                      uint64_t *d_frame_start, int32_t *d_status, void *stream);
+
 /* ---- several tracks, several devices (BASELINE configs[4]: a library of mixed 16/24-bit tracks) -----------
  * A PacketDecoder holds ONE cookie (decoder.go:79-87); a library batch mixes cookies. A library handle owns one
  * pipeline per device and decodes any mix of tracks in one call: every track is checked like

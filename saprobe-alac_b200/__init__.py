@@ -11,6 +11,8 @@ own tests (/root/reference/README.md:38-54):
     NewLibraryDecoder(devices).DecodeTracks(tracks)           NEW: many tracks of mixed cookies, sharded over devices
     NewDecoder(file bytes | file object) -> Decoder           decode.go:50
     Decoder.Read(n) / Seek(ns) / Format() / Duration() / Position()   decode.go:78-190
+    PacketDecoder.DecodePlanar(d_packed, d_offsets, d_sizes)  NEW: CUDA tensors in, channel-planar samples out (torch)
+    LoadTrack(file bytes | file object) -> (Tensor[C, T], PCMFormat)  NEW: NewDecoder(...).ReadAll() as a CUDA tensor
 
 Errors mirror errors.go:22-34: ErrConfig, ErrNoTrack, ErrDecode (exception classes; `.status` is the
 status word of the C ABI, `str()` the reference's wrapped message).
@@ -37,6 +39,7 @@ ST_OK = 0
 ST_INVALID_COOKIE, ST_UNSUPPORTED_VERSION, ST_UNSUPPORTED_ELEMENT, ST_INVALID_HEADER = 1, 2, 3, 4
 ST_INVALID_SHIFT, ST_BITSTREAM_OVERRUN, ST_SAMPLE_OVERRUN, ST_BIT_DEPTH = 5, 6, 7, 8
 ST_REF_PANIC, ST_UNSUPPORTED_CONFIG, ST_IO_TRUNCATED = 9, 10, 11
+SAMPLES_S16, SAMPLES_S32, SAMPLES_F32 = 1, 2, 3
 
 
 class PacketConfig(C.Structure):
@@ -125,6 +128,7 @@ def _load():
         'alacb200_library_devices': (C.c_int32, [vp]),
         'alacb200_library_decode_tracks': (C.c_int32, [vp, C.POINTER(TrackDesc), C.c_uint32]),
         'alacb200_decode_packets_device': (C.c_int32, [vp, vp, C.c_uint64, vp, vp, C.c_uint32, vp, C.c_uint64, vp, vp, vp]),
+        'alacb200_decode_planar_device': (C.c_int32, [vp, vp, C.c_uint64, vp, vp, C.c_uint32, C.c_int32, vp, C.c_uint64, vp, vp, vp]),
         'alacb200_pinned_alloc': (vp, [C.c_size_t]),
         'alacb200_pinned_free': (None, [vp]),
         'alacb200_strerror': (C.c_char_p, [C.c_int32]),
@@ -149,7 +153,7 @@ lib = _load()
 ABI_SYMBOLS = ('alacb200_parse_cookie alacb200_bytes_per_sample alacb200_create alacb200_destroy alacb200_format '
                'alacb200_get_config alacb200_max_packet_pcm_bytes alacb200_decode_packets alacb200_arena '
                'alacb200_library_create alacb200_library_destroy alacb200_library_devices '
-               'alacb200_library_decode_tracks alacb200_decode_packets_device alacb200_pinned_alloc alacb200_pinned_free alacb200_strerror '
+               'alacb200_library_decode_tracks alacb200_decode_packets_device alacb200_decode_planar_device alacb200_pinned_alloc alacb200_pinned_free alacb200_strerror '
                'alacb200_format_error alacb200_last_error alacb200_device_count alacb200_set_profiling '
                'alacb200_get_profile alacb200_mp4_find_alac_track alacb200_mp4_free_track alacb200_mp4_cookie '
                'alacb200_mp4_samples alacb200_mp4_error').split()
@@ -338,6 +342,38 @@ class PacketDecoder:
             raise errs[0]
         return pcm[0]
 
+    def DecodePlanar(self, d_packed, d_offsets, d_sizes, dtype=None):
+        """Device-resident batch -> channel-planar samples, enqueued on torch.cuda.current_stream() without a host
+        synchronisation. d_packed: uint8 CUDA tensor the packets live in (16-byte aligned, padded to a multiple of 16
+        bytes, every packet inside it); d_offsets: int64 [n]; d_sizes: int32 [n]; all on this decoder's device.
+        dtype: torch.float32 (default; full scale is [-1, 1)), torch.int32, or torch.int16 (16-bit streams only).
+        -> (samples [channels, n * frame_length], frame_start int64 [n + 1], status int32 [n]): packet i's frames are
+        samples[:, frame_start[i]:frame_start[i + 1]], a failed packet has none, frame_start[n] is the total, and
+        samples past the total are not written."""
+        import torch
+        dtype = torch.float32 if dtype is None else dtype
+        types = {torch.int16: SAMPLES_S16, torch.int32: SAMPLES_S32, torch.float32: SAMPLES_F32}
+        if dtype not in types:
+            raise ValueError(f'DecodePlanar: dtype must be torch.int16, torch.int32 or torch.float32, not {dtype}')
+        if dtype == torch.int16 and self.config.BitDepth != 16:
+            raise ValueError(f'DecodePlanar: torch.int16 holds 16-bit streams only, this one is {self.config.BitDepth}-bit')
+        dev = torch.device('cuda', self.device)
+        for name, t, want in (('d_packed', d_packed, torch.uint8), ('d_offsets', d_offsets, torch.int64), ('d_sizes', d_sizes, torch.int32)):
+            if t.device != dev or t.dtype != want or not t.is_contiguous():
+                raise ValueError(f'DecodePlanar: {name} must be a contiguous {want} tensor on {dev}')
+        n = d_sizes.numel()
+        if d_offsets.numel() != n:
+            raise ValueError('DecodePlanar: d_offsets and d_sizes differ in length')
+        with torch.cuda.device(dev):
+            samples = torch.empty((self.config.NumChannels, n * self.config.FrameLength), dtype=dtype, device=dev)
+            frame_start = torch.empty(n + 1, dtype=torch.int64, device=dev)
+            status = torch.empty(n, dtype=torch.int32, device=dev)
+            rc = lib.alacb200_decode_planar_device(self._h, d_packed.data_ptr(), d_packed.numel(), d_offsets.data_ptr(),
+                                                   d_sizes.data_ptr(), n, types[dtype], samples.data_ptr(), samples.shape[1],
+                                                   frame_start.data_ptr(), status.data_ptr(), torch.cuda.current_stream(dev).cuda_stream)
+        _check(rc, 'alacb200_decode_planar_device')
+        return samples, frame_start, status
+
     # -- profiling -----------------------------------------------------------------------------------
     def set_profiling(self, on: bool):
         _check(lib.alacb200_set_profiling(self._h, int(on)), 'alacb200_set_profiling')
@@ -474,6 +510,27 @@ def FindALACTrack(data: bytes):
 _NS = 1_000_000_000
 
 
+def _open_track(rs):
+    """NewDecoder's container steps (decode.go:50-60): -> (file bytes, PacketConfig, [(offset, size)])."""
+    data = rs if isinstance(rs, (bytes, bytearray, memoryview)) else rs.read()
+    data = bytes(data)
+    cookie, samples = FindALACTrack(data)
+    try:
+        config = ParseMagicCookie(cookie)
+    except AlacError as e:
+        e.args = ('parsing ALAC config: ' + e.args[0],)  # decode.go:58
+        raise
+    return data, config, samples
+
+
+def _packet_error(idx: int, status: int) -> AlacError:
+    """The error Read returns for packet idx that failed with `status` (decode.go:181)."""
+    item = error_from_status(status)
+    err = type(item)(f'decoding packet {idx}: {item.args[0]}')
+    err.status = item.status
+    return err
+
+
 class Decoder:
     """Streaming Decoder, decode.go:32-190, with a GPU read-ahead window behind Read/Seek.
 
@@ -484,14 +541,7 @@ class Decoder:
     """
 
     def __init__(self, rs, device: int = 0, window: int = 2048):
-        data = rs if isinstance(rs, (bytes, bytearray, memoryview)) else rs.read()
-        data = bytes(data)
-        cookie, samples = FindALACTrack(data)
-        try:
-            config = ParseMagicCookie(cookie)
-        except AlacError as e:
-            e.args = ('parsing ALAC config: ' + e.args[0],)  # decode.go:58
-            raise
+        data, config, samples = _open_track(rs)
         self.dec = NewPacketDecoder(config, device)
         # the file image lives in pinned memory for the life of the decoder: every window is read in place from it
         # (image + sample-table offsets straight to the C ABI, asynchronous H2D), nothing is re-packed
@@ -562,10 +612,7 @@ class Decoder:
         if st[k] == ST_IO_TRUNCATED:  # io.ReadFull failure, decode.go:172-174
             raise IOError(f'reading sample {idx}: unexpected EOF')
         if st[k] != ST_OK:
-            item = error_from_status(int(st[k]))
-            err = type(item)(f'decoding packet {idx}: {item.args[0]}')  # decode.go:181
-            err.status = item.status
-            raise err
+            raise _packet_error(idx, int(st[k]))
         self._buf, self._bufOff = out[k, :nb[k]].tobytes(), 0
         self.sampleIdx += 1
 
@@ -600,3 +647,46 @@ class Decoder:
 
 def NewDecoder(rs, device: int = 0, window: int = 2048) -> Decoder:
     return Decoder(rs, device, window)
+
+
+def LoadTrack(rs, device: int = 0, dtype=None):
+    """An M4A (bytes or a file object) as a channel-planar CUDA tensor: -> (samples [channels, frames] on cuda:device,
+    PCMFormat). The samples are exactly what NewDecoder(rs).ReadAll() returns, reinterpreted as dtype (see
+    PacketDecoder.DecodePlanar), and the errors are ReadAll's: ErrNoTrack, ErrConfig, ErrDecode for the first failing
+    packet, IOError when a sample lies outside the file, whichever comes first in packet order.
+
+    The file image and its sample table are uploaded once; the packets before the first sample outside the image are
+    decoded in one DecodePlanar call, and only the total frame count and the first failure come back to the host."""
+    import torch
+    data, config, samples = _open_track(rs)
+    dec = NewPacketDecoder(config, device)
+    try:
+        dev = torch.device('cuda', device)
+        n = len(samples)
+        offs = np.array([o for o, _ in samples], dtype=np.uint64).reshape(n)
+        sizes = np.array([z for _, z in samples], dtype=np.uint32).reshape(n)
+        size = np.uint64(len(data))
+        outside = (offs > size) | (sizes.astype(np.uint64) > size - np.minimum(offs, size))  # never handed to the kernel
+        n_ok = int(np.argmax(outside)) if outside.any() else n
+        padded = (len(data) + 15) // 16 * 16
+        host = torch.zeros(padded, dtype=torch.uint8, pin_memory=True)
+        host.numpy()[:len(data)] = np.frombuffer(data, dtype=np.uint8)
+        d_image = host.to(dev, non_blocking=True)
+        table = torch.from_numpy(np.concatenate([offs[:n_ok].view(np.int64), sizes[:n_ok].astype(np.int64)]))
+        d_table = table.to(dev)
+        with torch.cuda.device(dev):
+            pcm, frame_start, status = dec.DecodePlanar(d_image, d_table[:n_ok], d_table[n_ok:].to(torch.int32), dtype)
+            if n_ok:
+                failed = torch.where(status != 0, torch.arange(n_ok, device=dev, dtype=torch.int32), n_ok)
+                first = failed.min()
+                info = torch.stack([frame_start[n_ok], first.long(), status[first.long().clamp(max=n_ok - 1)].long()]).cpu().tolist()
+            else:
+                info = [0, 0, 0]
+        total, first_bad, first_status = info
+        if first_bad < n_ok:
+            raise _packet_error(first_bad, first_status)
+        if n_ok < n:
+            raise IOError(f'reading sample {n_ok}: unexpected EOF')  # io.ReadFull, decode.go:172-174
+        return pcm[:, :total], dec.Format()
+    finally:
+        dec.close()

@@ -1,9 +1,10 @@
-// alac_abi.cu -- the C ABI of include/alac_b200.h over the kernel in alac_kernels.cuh.
+// alac_abi.cu -- the C ABI of include/alac_b200.h over the kernels in alac_kernels.cuh and alac_planar.cuh.
 //
 // Host-side plumbing only: handles, device buffers, the chunked H2D -> decode kernel -> D2H pipeline over four slots (a
 // CUDA stream and its buffers each), the multi-track / multi-device front end, pinned memory, error text. No decode
 // arithmetic lives here and there is no CPU fallback: if CUDA is unusable every decode entry point fails.
 #include "alac_kernels.cuh"
+#include "alac_planar.cuh"
 
 #include <algorithm>
 #include <cstdio>
@@ -530,6 +531,16 @@ struct alacb200_library {
 
 namespace {
 
+// The device-path scratch is stream-ordered memory: moving to another stream first waits for the work of the previous one.
+int32_t use_device_path_stream(alacb200_decoder *dec, cudaStream_t st) {
+    if (st != dec->device_path_stream && dec->device_path_work.scratch.p) {
+        CU(cudaStreamSynchronize(dec->device_path_stream));
+        dec->device_path_work.release(dec->device_path_stream);
+    }
+    dec->device_path_stream = st;
+    return ALACB200_OK;
+}
+
 // The tracks `order` on one device: already grouped by kernel config (so every launch is depth-homogeneous, SURVEY.md
 // 8e), cut into pipeline chunks that may span several tracks.
 int32_t decode_tracks_on(Pipeline &pipe, alacb200_track_desc *tracks, const std::vector<Shape> &shapes, const std::vector<uint32_t> &order) {
@@ -691,15 +702,66 @@ int32_t alacb200_decode_packets_device(alacb200_decoder *dec, const uint8_t *d_p
     }
     DeviceGuard guard(dec->pipe.device);
     if (!guard.ok) return ALACB200_E_CUDA;
-    // the scratch is stream-ordered memory: moving to another stream first waits for the work of the previous one
     cudaStream_t st = (cudaStream_t)stream;
-    if (st != dec->device_path_stream && dec->device_path_work.scratch.p) {
-        CU(cudaStreamSynchronize(dec->device_path_stream));
-        dec->device_path_work.release(dec->device_path_stream);
-    }
-    dec->device_path_stream = st;
+    const int32_t rc = use_device_path_stream(dec, st);
+    if (rc != ALACB200_OK) return rc;
     return dec->pipe.launch(dec->device_path_work, dec->shape, d_packed, d_offsets, d_sizes, n, d_pcm_out, out_stride, d_out_bytes,
                             d_status, st);
+}
+
+int32_t alacb200_decode_planar_device(alacb200_decoder *dec, const uint8_t *d_packed, uint64_t packed_bytes,
+                                      const uint64_t *d_offsets, const uint32_t *d_sizes, uint32_t n, int32_t sample_type,
+                                      void *d_out, uint64_t channel_stride, uint64_t *d_frame_start, int32_t *d_status,
+                                      void *stream) {
+    (void)packed_bytes;
+    if (!dec) return ALACB200_E_ARG;
+    const size_t esz = sample_type == ALACB200_SAMPLES_S16 ? 2 : (sample_type == ALACB200_SAMPLES_S32 || sample_type == ALACB200_SAMPLES_F32) ? 4 : 0;
+    if (esz == 0 || (sample_type == ALACB200_SAMPLES_S16 && dec->cfg.bit_depth != 16)) {
+        g_last_error = "sample_type must be S16 (16-bit streams only), S32 or F32";
+        return ALACB200_E_ARG;
+    }
+    if (!d_frame_start) return ALACB200_E_ARG;
+    const uint32_t fl = dec->cfg.frame_length, bpf = dec->shape.dev.num_channels * dec->shape.dev.bps;
+    if (n && (!d_packed || !d_offsets || !d_sizes || !d_out || !d_status)) return ALACB200_E_ARG;
+    if (channel_stride < (uint64_t)n * fl || (((uintptr_t)d_out) % esz) || (((uintptr_t)d_packed) & 15u)) {
+        g_last_error = "channel_stride must be >= n * frame_length; d_out aligned to its element size; d_packed 16-byte aligned";
+        return ALACB200_E_ARG;
+    }
+    DeviceGuard guard(dec->pipe.device);
+    if (!guard.ok) return ALACB200_E_CUDA;
+    cudaStream_t st = (cudaStream_t)stream;
+    if (n == 0) {
+        CU(cudaMemsetAsync(d_frame_start, 0, sizeof(uint64_t), st));
+        return ALACB200_OK;
+    }
+    int32_t rc = use_device_path_stream(dec, st);
+    if (rc != ALACB200_OK) return rc;
+    // the interleaved intermediate: packet slots of frame_bytes rounded up to 16, then out_bytes[n]; freed on the stream
+    // at the end of the call
+    const uint64_t slot = (dec->shape.frame_bytes + 15u) / 16u * 16u;
+    uint8_t *inter = nullptr;
+    if (pool_alloc((void **)&inter, (size_t)(n * slot + (uint64_t)n * 4u), st) != cudaSuccess) {
+        g_last_error = "cudaMallocAsync failed (planar intermediate)";
+        cudaGetLastError();
+        return ALACB200_E_NOMEM;
+    }
+    uint32_t *d_out_bytes = (uint32_t *)(inter + n * slot);
+    rc = dec->pipe.launch(dec->device_path_work, dec->shape, d_packed, d_offsets, d_sizes, n, inter, slot, d_out_bytes, d_status, st);
+    if (rc == ALACB200_OK) {
+        alac_frame_scan_kernel<<<1, SCAN_THREADS, 0, st>>>(d_out_bytes, d_status, n, bpf, d_frame_start);
+        const uint32_t tile = planar_tile_frames(bpf, fl);
+        const dim3 grid(n, (fl + tile - 1) / tile);
+        const uint32_t ch = dec->shape.dev.num_channels, bps = dec->shape.dev.bps;
+        if (sample_type == ALACB200_SAMPLES_S16)
+            alac_planar_kernel<int16_t><<<grid, PLANAR_THREADS, 0, st>>>(inter, slot, d_frame_start, ch, bps, tile, (int16_t *)d_out, channel_stride);
+        else if (sample_type == ALACB200_SAMPLES_S32)
+            alac_planar_kernel<int32_t><<<grid, PLANAR_THREADS, 0, st>>>(inter, slot, d_frame_start, ch, bps, tile, (int32_t *)d_out, channel_stride);
+        else
+            alac_planar_kernel<float><<<grid, PLANAR_THREADS, 0, st>>>(inter, slot, d_frame_start, ch, bps, tile, (float *)d_out, channel_stride);
+        if (!cuda_ok(cudaGetLastError(), "alac_planar_kernel")) rc = ALACB200_E_CUDA;
+    }
+    cudaFreeAsync(inter, st);
+    return rc;
 }
 
 int32_t alacb200_decode_packets(alacb200_decoder *dec, const uint8_t *packed, uint64_t packed_bytes, const uint64_t *offsets,
