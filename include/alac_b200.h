@@ -203,6 +203,49 @@ int32_t alacb200_library_devices(const alacb200_library *lib);
  * the first device error. One call at a time per library. */
 int32_t alacb200_library_decode_tracks(alacb200_library *lib, alacb200_track_desc *tracks, uint32_t ntracks);
 
+/* Many tracks of any mix of cookies on DEVICE buffers into channel-planar samples, on one device of the library
+ * (alacb200_library_decode_planar_device): the multi-track form of alacb200_decode_planar_device. */
+typedef struct alacb200_planar_track {
+    /* in */
+    const uint8_t *cookie;   /* magic cookie of the track (with or without the frma/alac wrappers) */
+    size_t cookie_len;
+    uint32_t n;              /* this track's rows of the shared packet table: rows follow track order, track 0 first */
+    uint32_t reserved;
+    void *d_out;             /* num_channels rows of channel_stride elements of the sample type */
+    uint64_t channel_stride; /* >= n*frame_length of THIS track (elements) */
+    /* out */
+    alacb200_config config;  /* the parsed cookie */
+    int32_t track_status;    /* ALACB200_ST_OK, or why the track has no decoder (INVALID_COOKIE ... UNSUPPORTED_CONFIG) */
+    int32_t result;          /* ALACB200_OK or ALACB200_E_CONFIG (see track_status) */
+} alacb200_planar_track;
+/* The packet table (d_offsets, d_sizes, d_status) has N = sum of n rows, track after track; offsets are absolute in
+ * d_packed, which follows the rules of alacb200_decode_packets_device (16-byte aligned, readable for packed_bytes rounded
+ * up to 16). Track t's rows are [r_t, r_t + n_t) with r_t the sum of the earlier n; packet r_t + i lands in
+ * d_out_t[c*channel_stride_t + fs[i] .. fs[i+1]) of every channel c, where fs = d_frame_start + r_t + t holds the
+ * track's n_t + 1 frame starts ([n_t] is its total). d_frame_start therefore has N + ntracks entries. A failed packet
+ * contributes no frames; frames between a track's total and its channel_stride are not written.
+ *
+ * A track whose cookie fails ParseMagicCookie + NewPacketDecoder's checks gets result ALACB200_E_CONFIG: its rows get
+ * track_status as their status word, its frame starts are 0 and nothing is written to its d_out. The other tracks are
+ * cut into maximal runs of adjacent tracks of one kernel config (frame length, depth, channels, pb/mb/kb), and every
+ * run is one decode launch, one frame scan and one planar pass; a table ordered by config is one decode launch per
+ * config. Enqueued on `stream` without synchronising the host (except the stream switch of the device scratch, as
+ * for alacb200_decode_packets_device). A run's interleaved intermediate (its rows of max_packet_pcm_bytes rounded up to
+ * 16, plus 4 bytes a row) comes from the device's stream-ordered pool and is freed on the stream after the run, so the
+ * peak is the largest run's. The track table goes through pinned staging that is not written again before its copy
+ * has completed.
+ *
+ * ntracks == 0 or N == 0 writes only the frame starts, all 0. ALACB200_E_ARG, with nothing enqueued, for an unknown
+ * sample_type, S16 with a decodable track that is not 16-bit, a decodable track with n > 0 whose channel_stride is
+ * below n*frame_length or whose d_out is NULL or not aligned to its element size, a misaligned d_packed, a NULL
+ * pointer (d_packed, d_offsets, d_sizes and d_status may be NULL when N == 0), more than 2^32-1 rows, or a device that
+ * is not one of the library's. One call at a time per library. */
+int32_t alacb200_library_decode_planar_device(alacb200_library *lib, int device, const uint8_t *d_packed,
+                                              uint64_t packed_bytes, const uint64_t *d_offsets,
+                                              const uint32_t *d_sizes, alacb200_planar_track *tracks,
+                                              uint32_t ntracks, int32_t sample_type, uint64_t *d_frame_start,
+                                              int32_t *d_status, void *stream);
+
 /* Pinned (page-locked) host memory for packed input / PCM output. */
 void *alacb200_pinned_alloc(size_t bytes);
 void alacb200_pinned_free(void *p);

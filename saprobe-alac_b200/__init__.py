@@ -13,6 +13,8 @@ own tests (/root/reference/README.md:38-54):
     Decoder.Read(n) / Seek(ns) / Format() / Duration() / Position()   decode.go:78-190
     PacketDecoder.DecodePlanar(d_packed, d_offsets, d_sizes)  NEW: CUDA tensors in, channel-planar samples out (torch)
     LoadTrack(file bytes | file object) -> (Tensor[C, T], PCMFormat)  NEW: NewDecoder(...).ReadAll() as a CUDA tensor
+    LibraryDecoder.DecodePlanar(d_packed, ..., cookies, counts)  NEW: many tracks of mixed cookies, device-resident (torch)
+    LoadTracks([file bytes | file object]) -> [LoadedTrack]    NEW: LoadTrack of many files in one decode call
 
 Errors mirror errors.go:22-34: ErrConfig, ErrNoTrack, ErrDecode (exception classes; `.status` is the
 status word of the C ABI, `str()` the reference's wrapped message).
@@ -78,6 +80,13 @@ class TrackDesc(C.Structure):
                 ('reserved2', C.c_int32)]
 
 
+class PlanarTrackDesc(C.Structure):
+    """alacb200_planar_track (include/alac_b200.h): one track of a multi-track planar call."""
+    _fields_ = [('cookie', C.c_void_p), ('cookie_len', C.c_size_t), ('n', C.c_uint32), ('reserved', C.c_uint32),
+                ('d_out', C.c_void_p), ('channel_stride', C.c_uint64), ('config', PacketConfig), ('track_status', C.c_int32),
+                ('result', C.c_int32)]
+
+
 class SampleInfo(C.Structure):
     """SampleInfo, internal/mp4/mp4.go:28-31."""
     _fields_ = [('Offset', C.c_uint64), ('Size', C.c_uint32), ('_reserved', C.c_uint32)]
@@ -129,6 +138,8 @@ def _load():
         'alacb200_library_decode_tracks': (C.c_int32, [vp, C.POINTER(TrackDesc), C.c_uint32]),
         'alacb200_decode_packets_device': (C.c_int32, [vp, vp, C.c_uint64, vp, vp, C.c_uint32, vp, C.c_uint64, vp, vp, vp]),
         'alacb200_decode_planar_device': (C.c_int32, [vp, vp, C.c_uint64, vp, vp, C.c_uint32, C.c_int32, vp, C.c_uint64, vp, vp, vp]),
+        'alacb200_library_decode_planar_device': (C.c_int32, [vp, C.c_int, vp, C.c_uint64, vp, vp, C.POINTER(PlanarTrackDesc),
+                                                              C.c_uint32, C.c_int32, vp, vp, vp]),
         'alacb200_pinned_alloc': (vp, [C.c_size_t]),
         'alacb200_pinned_free': (None, [vp]),
         'alacb200_strerror': (C.c_char_p, [C.c_int32]),
@@ -153,7 +164,8 @@ lib = _load()
 ABI_SYMBOLS = ('alacb200_parse_cookie alacb200_bytes_per_sample alacb200_create alacb200_destroy alacb200_format '
                'alacb200_get_config alacb200_max_packet_pcm_bytes alacb200_decode_packets alacb200_arena '
                'alacb200_library_create alacb200_library_destroy alacb200_library_devices '
-               'alacb200_library_decode_tracks alacb200_decode_packets_device alacb200_decode_planar_device alacb200_pinned_alloc alacb200_pinned_free alacb200_strerror '
+               'alacb200_library_decode_tracks alacb200_decode_packets_device alacb200_decode_planar_device '
+               'alacb200_library_decode_planar_device alacb200_pinned_alloc alacb200_pinned_free alacb200_strerror '
                'alacb200_format_error alacb200_last_error alacb200_device_count alacb200_set_profiling '
                'alacb200_get_profile alacb200_mp4_find_alac_track alacb200_mp4_free_track alacb200_mp4_cookie '
                'alacb200_mp4_samples alacb200_mp4_error').split()
@@ -176,6 +188,44 @@ def error_from_status(status: int, prefix: str = '') -> AlacError:
 def _check(rc: int, what: str):
     if rc != OK:
         raise CudaError(f'{what} failed (rc={rc}): {lib.alacb200_last_error().decode()}')
+
+
+def _config_status(config: PacketConfig) -> int:
+    """NewPacketDecoder's checks of a parsed cookie (decoder.go:90-110): ST_OK or the status it fails with."""
+    if lib.alacb200_bytes_per_sample(config.BitDepth) == 0:
+        return ST_BIT_DEPTH
+    if not (1 <= config.NumChannels <= 8 and 1 <= config.FrameLength <= 65536):
+        return ST_UNSUPPORTED_CONFIG
+    return ST_OK
+
+
+def _config_error(status: int, config: PacketConfig) -> AlacError:
+    """The error NewPacketDecoder raises for a cookie that fails its checks with `status`."""
+    err = error_from_status(status)
+    if status == ST_BIT_DEPTH:
+        err.args = (f'{err.args[0]}: {config.BitDepth}',)  # decoder.go:92
+    return err
+
+
+def _planar_type(torch, dtype, bit_depths=()):
+    """dtype (None: float32) -> (torch dtype, SAMPLES_*), or ValueError for a dtype the planar path does not produce or
+    int16 for a stream that is not 16-bit."""
+    dtype = torch.float32 if dtype is None else dtype
+    types = {torch.int16: SAMPLES_S16, torch.int32: SAMPLES_S32, torch.float32: SAMPLES_F32}
+    if dtype not in types:
+        raise ValueError(f'DecodePlanar: dtype must be torch.int16, torch.int32 or torch.float32, not {dtype}')
+    for bits in bit_depths:
+        if dtype == torch.int16 and bits != 16:
+            raise ValueError(f'DecodePlanar: torch.int16 holds 16-bit streams only, this one is {bits}-bit')
+    return dtype, types[dtype]
+
+
+def _check_device_tensors(who, dev, **tensors):
+    import torch
+    want = {'d_packed': torch.uint8, 'd_offsets': torch.int64, 'd_sizes': torch.int32}
+    for name, t in tensors.items():
+        if t.device != dev or t.dtype != want[name] or not t.is_contiguous():
+            raise ValueError(f'{who}: {name} must be a contiguous {want[name]} tensor on {dev}')
 
 
 # ---- config.go ----------------------------------------------------------------------------------------
@@ -239,10 +289,7 @@ class PacketDecoder:
         st = C.c_int32(0)
         rc = lib.alacb200_create(C.byref(config), device, C.byref(self._h), C.byref(st))
         if rc == E_CONFIG:
-            err = error_from_status(st.value)
-            if st.value == ST_BIT_DEPTH:
-                err.args = (f'{err.args[0]}: {config.BitDepth}',)  # decoder.go:92
-            raise err
+            raise _config_error(st.value, config)
         _check(rc, 'alacb200_create')
         self.config = config
         self.device = device
@@ -351,16 +398,9 @@ class PacketDecoder:
         samples[:, frame_start[i]:frame_start[i + 1]], a failed packet has none, frame_start[n] is the total, and
         samples past the total are not written."""
         import torch
-        dtype = torch.float32 if dtype is None else dtype
-        types = {torch.int16: SAMPLES_S16, torch.int32: SAMPLES_S32, torch.float32: SAMPLES_F32}
-        if dtype not in types:
-            raise ValueError(f'DecodePlanar: dtype must be torch.int16, torch.int32 or torch.float32, not {dtype}')
-        if dtype == torch.int16 and self.config.BitDepth != 16:
-            raise ValueError(f'DecodePlanar: torch.int16 holds 16-bit streams only, this one is {self.config.BitDepth}-bit')
+        dtype, sample_type = _planar_type(torch, dtype, (self.config.BitDepth,))
         dev = torch.device('cuda', self.device)
-        for name, t, want in (('d_packed', d_packed, torch.uint8), ('d_offsets', d_offsets, torch.int64), ('d_sizes', d_sizes, torch.int32)):
-            if t.device != dev or t.dtype != want or not t.is_contiguous():
-                raise ValueError(f'DecodePlanar: {name} must be a contiguous {want} tensor on {dev}')
+        _check_device_tensors('DecodePlanar', dev, d_packed=d_packed, d_offsets=d_offsets, d_sizes=d_sizes)
         n = d_sizes.numel()
         if d_offsets.numel() != n:
             raise ValueError('DecodePlanar: d_offsets and d_sizes differ in length')
@@ -369,7 +409,7 @@ class PacketDecoder:
             frame_start = torch.empty(n + 1, dtype=torch.int64, device=dev)
             status = torch.empty(n, dtype=torch.int32, device=dev)
             rc = lib.alacb200_decode_planar_device(self._h, d_packed.data_ptr(), d_packed.numel(), d_offsets.data_ptr(),
-                                                   d_sizes.data_ptr(), n, types[dtype], samples.data_ptr(), samples.shape[1],
+                                                   d_sizes.data_ptr(), n, sample_type, samples.data_ptr(), samples.shape[1],
                                                    frame_start.data_ptr(), status.data_ptr(), torch.cuda.current_stream(dev).cuda_stream)
         _check(rc, 'alacb200_decode_planar_device')
         return samples, frame_start, status
@@ -454,7 +494,7 @@ class LibraryDecoder:
             st = lib.alacb200_parse_cookie(bytes(tr.cookie) if tr.cookie is not None else b'', len(cookie), C.byref(cfg))
             bps = lib.alacb200_bytes_per_sample(cfg.BitDepth) if st == ST_OK else 0
             stride = (cfg.FrameLength * cfg.NumChannels * bps + 3) // 4 * 4 if bps else 4
-            ok_shape = bps and 1 <= cfg.NumChannels <= 8 and 1 <= cfg.FrameLength <= 65536
+            ok_shape = st == ST_OK and _config_status(cfg) == ST_OK
             pcm = out[t] if out is not None else (np.zeros((n, stride), dtype=np.uint8) if ok_shape else np.zeros((0, 4), dtype=np.uint8))
             nb = np.zeros(n, dtype=np.uint32)
             stt = np.zeros(n, dtype=np.int32)
@@ -472,13 +512,72 @@ class LibraryDecoder:
             r.config = PacketConfig.from_buffer_copy(d.config)
             r.device = d.device
             if d.result == E_CONFIG:
-                r.err = error_from_status(d.track_status)
-                if d.track_status == ST_BIT_DEPTH:
-                    r.err.args = (f'{r.err.args[0]}: {r.config.BitDepth}',)  # decoder.go:92
+                r.err = _config_error(d.track_status, r.config)
             elif d.result != OK:
                 r.err = CudaError(f'track {t}: rc={d.result}')
         del keep
         return results
+
+    def DecodePlanar(self, d_packed, d_offsets, d_sizes, cookies, counts, dtype=None, device=None):
+        """Device-resident packets of many tracks -> channel-planar samples per track, enqueued on
+        torch.cuda.current_stream() without a host synchronisation: the multi-track PacketDecoder.DecodePlanar.
+
+        The packet table is shared: d_offsets int64 [N] (absolute in d_packed), d_sizes int32 [N], track t owning the
+        next counts[t] rows, track 0 first; d_packed as for PacketDecoder.DecodePlanar; all on cuda:device (default: the
+        library's first device, which must be one of its devices). cookies[t] is track t's magic cookie. Adjacent
+        tracks of one kernel config share their launches, so a table ordered by config is one decode launch per config.
+        -> (samples, frame_start int64 [N + T], status int32 [N], errors):
+          samples[t]   [channels_t, counts[t] * frame_length_t] of dtype, or None for a track whose cookie fails
+                       ParseMagicCookie + NewPacketDecoder (its error is errors[t], as LibraryDecoder.DecodeTracks
+                       reports it; its rows get that status word). All tracks' samples are views of one allocation.
+          frame_start  track t's counts[t] + 1 entries start at (its first row + t): its packet i's frames are
+                       samples[t][:, fs[i]:fs[i + 1]], a failed packet has none, fs[counts[t]] is its total, and
+                       samples past the total are not written."""
+        import torch
+        device = self.devices[0] if device is None else device
+        dtype, sample_type = _planar_type(torch, dtype)
+        dev = torch.device('cuda', device)
+        _check_device_tensors('LibraryDecoder.DecodePlanar', dev, d_packed=d_packed, d_offsets=d_offsets, d_sizes=d_sizes)
+        counts = [int(c) for c in counts]
+        nt, rows = len(cookies), sum(counts)
+        if len(counts) != nt or d_offsets.numel() != rows or d_sizes.numel() != rows:
+            raise ValueError('LibraryDecoder.DecodePlanar: one count per cookie, and sum(counts) rows in d_offsets and d_sizes')
+        descs = (PlanarTrackDesc * max(nt, 1))()
+        cookies = [np.frombuffer(bytes(c) if c is not None else b'', dtype=np.uint8) for c in cookies]
+        esz = torch.empty((), dtype=dtype).element_size()
+        spans, total = [], 0  # per track: (first element, channels, channel stride) of its samples in one allocation
+        for t in range(nt):
+            cfg = PacketConfig()
+            ok = lib.alacb200_parse_cookie(cookies[t].tobytes(), len(cookies[t]), C.byref(cfg)) == ST_OK and _config_status(cfg) == ST_OK
+            stride = counts[t] * cfg.FrameLength if ok else 0
+            spans.append((total, cfg.NumChannels if ok else 0, stride))
+            total += -(-cfg.NumChannels * stride * esz // 16) * 16 // esz if ok else 0  # every track starts 16-byte aligned
+        with torch.cuda.device(dev):
+            flat = torch.empty(max(total, 1), dtype=dtype, device=dev)
+            frame_start = torch.empty(rows + nt, dtype=torch.int64, device=dev)
+            status = torch.empty(rows, dtype=torch.int32, device=dev)
+            for t in range(nt):
+                d = descs[t]
+                d.cookie, d.cookie_len = cookies[t].ctypes.data if len(cookies[t]) else None, len(cookies[t])
+                d.n, d.channel_stride = counts[t], spans[t][2]
+                d.d_out = flat.data_ptr() + spans[t][0] * esz
+            rc = lib.alacb200_library_decode_planar_device(self._h, device, d_packed.data_ptr(), d_packed.numel(), d_offsets.data_ptr(),
+                                                           d_sizes.data_ptr(), descs, nt, sample_type, frame_start.data_ptr(),
+                                                           status.data_ptr(), torch.cuda.current_stream(dev).cuda_stream)
+        if rc == E_ARG:
+            raise ValueError(f'LibraryDecoder.DecodePlanar: {lib.alacb200_last_error().decode()}')
+        _check(rc, 'alacb200_library_decode_planar_device')
+        samples, errors = [], []
+        for t in range(nt):
+            d = descs[t]
+            if d.result == E_CONFIG:
+                samples.append(None)
+                errors.append(_config_error(d.track_status, PacketConfig.from_buffer_copy(d.config)))
+            else:
+                a, ch, stride = spans[t]
+                samples.append(flat[a:a + ch * stride].view(ch, stride))
+                errors.append(None)
+        return samples, frame_start, status, errors
 
 
 def NewLibraryDecoder(devices=(0,)) -> LibraryDecoder:
@@ -511,7 +610,7 @@ _NS = 1_000_000_000
 
 
 def _open_track(rs):
-    """NewDecoder's container steps (decode.go:50-60): -> (file bytes, PacketConfig, [(offset, size)])."""
+    """NewDecoder's container steps (decode.go:50-60): -> (file bytes, PacketConfig, [(offset, size)], cookie)."""
     data = rs if isinstance(rs, (bytes, bytearray, memoryview)) else rs.read()
     data = bytes(data)
     cookie, samples = FindALACTrack(data)
@@ -520,7 +619,7 @@ def _open_track(rs):
     except AlacError as e:
         e.args = ('parsing ALAC config: ' + e.args[0],)  # decode.go:58
         raise
-    return data, config, samples
+    return data, config, samples, cookie
 
 
 def _packet_error(idx: int, status: int) -> AlacError:
@@ -541,7 +640,7 @@ class Decoder:
     """
 
     def __init__(self, rs, device: int = 0, window: int = 2048):
-        data, config, samples = _open_track(rs)
+        data, config, samples, _ = _open_track(rs)
         self.dec = NewPacketDecoder(config, device)
         # the file image lives in pinned memory for the life of the decoder: every window is read in place from it
         # (image + sample-table offsets straight to the C ABI, asynchronous H2D), nothing is re-packed
@@ -649,44 +748,116 @@ def NewDecoder(rs, device: int = 0, window: int = 2048) -> Decoder:
     return Decoder(rs, device, window)
 
 
+@dataclass
+class LoadedTrack:
+    """One element of LoadTracks: samples [channels, frames] on the device and the PCMFormat, or the error."""
+    samples: object = None  # torch.Tensor
+    format: PCMFormat = None
+    err: Exception = None
+
+
+def LoadTracks(files, device: int = 0, dtype=None):
+    """Many M4A files (bytes or file objects) as channel-planar CUDA tensors in one decode call: -> [LoadedTrack].
+    Element t is what LoadTrack(files[t], device, dtype) returns (samples, format) or raises (err): the same values,
+    shape, dtype and device, the same exception type, text and status. One bad file does not fail the others.
+
+    The containers are parsed on the host; a track's packets from the first sample outside its file on are not
+    decoded (that sample is its IOError). The decodable tracks are ordered by kernel config, their images and sample
+    tables are uploaded through one pinned buffer in one copy, and one LibraryDecoder.DecodePlanar call decodes them.
+    One [T, 3] array comes back: each track's frame total, first failing packet and its status word, reduced per track
+    on the device. The samples of all tracks are views of one allocation."""
+    import torch
+    dev = torch.device('cuda', device)
+    out = [LoadedTrack() for _ in files]
+    todo = []  # (t, data, config, cookie, offsets, sizes, packets before the first one outside the file)
+    for t, rs in enumerate(files):
+        try:
+            data, config, samples, cookie = _open_track(rs)
+            st = _config_status(config)
+            if st != ST_OK:
+                raise _config_error(st, config)
+            _planar_type(torch, dtype, (config.BitDepth,))
+        except Exception as e:  # noqa: BLE001 -- the element's error, exactly what LoadTrack raises
+            out[t].err = e
+            continue
+        n = len(samples)
+        offs = np.array([o for o, _ in samples], dtype=np.uint64).reshape(n)
+        sizes = np.array([z for _, z in samples], dtype=np.uint32).reshape(n)
+        size = np.uint64(len(data))
+        outside = (offs > size) | (sizes.astype(np.uint64) > size - np.minimum(offs, size))  # never handed to the kernel
+        todo.append((t, data, config, cookie, offs, sizes, int(np.argmax(outside)) if outside.any() else n))
+    if not todo:
+        return out
+    todo.sort(key=lambda x: (x[2].BitDepth, x[2].NumChannels, x[2].FrameLength, x[2].PB, x[2].MB, x[2].KB))
+    # one pinned buffer, one copy: the images (each 16-byte aligned), then offsets i64 [N], sizes i32 [N], the row's
+    # track i32 [N], the row's packet index in its track i32 [N], and each track's total in frame_start i64 [T]
+    nt = len(todo)
+    counts = np.array([x[6] for x in todo], dtype=np.int64)
+    rows = int(counts.sum())
+    bases = np.zeros(nt, dtype=np.int64)
+    pos = 0
+    for k, x in enumerate(todo):
+        bases[k] = pos
+        pos += (len(x[1]) + 15) // 16 * 16
+    img = max(pos, 16)
+    size16 = lambda b: (int(b) + 15) // 16 * 16  # noqa: E731
+    at = [img]
+    for b in (8 * rows, 4 * rows, 4 * rows, 4 * rows):
+        at.append(size16(at[-1] + b))
+    host = torch.empty(size16(at[-1] + 8 * nt), dtype=torch.uint8, pin_memory=True)
+    h = host.numpy()
+    first_row = np.concatenate([[0], np.cumsum(counts)[:-1]]).astype(np.int64)
+    for k, x in enumerate(todo):
+        h[bases[k]:bases[k] + len(x[1])] = np.frombuffer(x[1], dtype=np.uint8)
+        a = first_row[k]
+        h[at[0] + 8 * a:at[0] + 8 * (a + counts[k])].view(np.int64)[:] = x[4][:counts[k]].view(np.int64) + bases[k]
+        h[at[1] + 4 * a:at[1] + 4 * (a + counts[k])].view(np.uint32)[:] = x[5][:counts[k]]
+    h[at[2]:at[2] + 4 * rows].view(np.int32)[:] = np.repeat(np.arange(nt, dtype=np.int32), counts)
+    h[at[3]:at[3] + 4 * rows].view(np.int32)[:] = np.arange(rows, dtype=np.int32) - np.repeat(first_row, counts).astype(np.int32)
+    h[at[4]:at[4] + 8 * nt].view(np.int64)[:] = first_row + counts + np.arange(nt)
+    lib_dec = LibraryDecoder((device,))
+    try:
+        with torch.cuda.device(dev):
+            d = host.to(dev, non_blocking=True)
+            d_offsets = d[at[0]:at[0] + 8 * rows].view(torch.int64)
+            d_sizes = d[at[1]:at[1] + 4 * rows].view(torch.int32)
+            track = d[at[2]:at[2] + 4 * rows].view(torch.int32).long()
+            index = d[at[3]:at[3] + 4 * rows].view(torch.int32).long()
+            totals_at = d[at[4]:at[4] + 8 * nt].view(torch.int64)
+            pcm, frame_start, status, errors = lib_dec.DecodePlanar(d[:img], d_offsets, d_sizes, [x[3] for x in todo], counts,
+                                                                    dtype, device)
+            # per track, the first failing packet and its status in one key: index << 32 | status, minimum over the track
+            none = torch.iinfo(torch.int64).max
+            key = torch.where(status != 0, (index << 32) | (status.long() & 0xffffffff), none)
+            first = torch.full((nt,), none, dtype=torch.int64, device=dev).scatter_reduce_(0, track, key, 'amin')
+            info = torch.stack([frame_start[totals_at], first >> 32, first & 0xffffffff], 1).cpu().tolist()
+    finally:
+        lib_dec.close()
+    for k, x in enumerate(todo):
+        t, config, n, n_ok = x[0], x[2], len(x[4]), x[6]
+        total, first_bad, first_status = info[k]
+        if errors[k] is not None:
+            out[t].err = errors[k]
+        elif first_bad < n_ok:
+            out[t].err = _packet_error(first_bad, first_status)
+        elif n_ok < n:
+            out[t].err = IOError(f'reading sample {n_ok}: unexpected EOF')  # io.ReadFull, decode.go:172-174
+        else:
+            out[t].samples = pcm[k][:, :total]
+            out[t].format = PCMFormat(config.SampleRate, config.BitDepth, config.NumChannels)
+    return out
+
+
 def LoadTrack(rs, device: int = 0, dtype=None):
     """An M4A (bytes or a file object) as a channel-planar CUDA tensor: -> (samples [channels, frames] on cuda:device,
     PCMFormat). The samples are exactly what NewDecoder(rs).ReadAll() returns, reinterpreted as dtype (see
     PacketDecoder.DecodePlanar), and the errors are ReadAll's: ErrNoTrack, ErrConfig, ErrDecode for the first failing
     packet, IOError when a sample lies outside the file, whichever comes first in packet order.
 
-    The file image and its sample table are uploaded once; the packets before the first sample outside the image are
-    decoded in one DecodePlanar call, and only the total frame count and the first failure come back to the host."""
-    import torch
-    data, config, samples = _open_track(rs)
-    dec = NewPacketDecoder(config, device)
-    try:
-        dev = torch.device('cuda', device)
-        n = len(samples)
-        offs = np.array([o for o, _ in samples], dtype=np.uint64).reshape(n)
-        sizes = np.array([z for _, z in samples], dtype=np.uint32).reshape(n)
-        size = np.uint64(len(data))
-        outside = (offs > size) | (sizes.astype(np.uint64) > size - np.minimum(offs, size))  # never handed to the kernel
-        n_ok = int(np.argmax(outside)) if outside.any() else n
-        padded = (len(data) + 15) // 16 * 16
-        host = torch.zeros(padded, dtype=torch.uint8, pin_memory=True)
-        host.numpy()[:len(data)] = np.frombuffer(data, dtype=np.uint8)
-        d_image = host.to(dev, non_blocking=True)
-        table = torch.from_numpy(np.concatenate([offs[:n_ok].view(np.int64), sizes[:n_ok].astype(np.int64)]))
-        d_table = table.to(dev)
-        with torch.cuda.device(dev):
-            pcm, frame_start, status = dec.DecodePlanar(d_image, d_table[:n_ok], d_table[n_ok:].to(torch.int32), dtype)
-            if n_ok:
-                failed = torch.where(status != 0, torch.arange(n_ok, device=dev, dtype=torch.int32), n_ok)
-                first = failed.min()
-                info = torch.stack([frame_start[n_ok], first.long(), status[first.long().clamp(max=n_ok - 1)].long()]).cpu().tolist()
-            else:
-                info = [0, 0, 0]
-        total, first_bad, first_status = info
-        if first_bad < n_ok:
-            raise _packet_error(first_bad, first_status)
-        if n_ok < n:
-            raise IOError(f'reading sample {n_ok}: unexpected EOF')  # io.ReadFull, decode.go:172-174
-        return pcm[:, :total], dec.Format()
-    finally:
-        dec.close()
+    LoadTracks([rs], device, dtype)[0]: the file image and its sample table are uploaded once, the packets before the
+    first sample outside the image are decoded in one call, and only the total frame count and the first failure come
+    back to the host."""
+    r = LoadTracks([rs], device, dtype)[0]
+    if r.err is not None:
+        raise r.err
+    return r.samples, r.format

@@ -193,6 +193,57 @@ struct Work {
     }
 };
 
+// The scratch of the device entry points, which enqueue on the caller's stream. It is stream-ordered memory: moving to
+// another stream first waits for the work of the previous one (the only host synchronisation of those entry points).
+struct DevicePathWork {
+    Work work;
+    cudaStream_t stream = nullptr;  // stream `work` was last used (and is owned) on
+    int32_t use(cudaStream_t st) {
+        if (st != stream && work.scratch.p) {
+            CU(cudaStreamSynchronize(stream));
+            work.release(stream);
+        }
+        stream = st;
+        return ALACB200_OK;
+    }
+};
+
+// Pinned staging of the small tables the device entry points upload (the planar path's track table). A buffer is
+// written again only once the copy that read it has completed, and a call never waits for that: it takes a buffer
+// whose copy is done, or adds one.
+struct TableStaging {
+    struct Buf {
+        PinBuf pin;
+        cudaEvent_t copied = nullptr;
+    };
+    std::vector<std::unique_ptr<Buf>> bufs;
+    int32_t upload(void *dst, const void *src, size_t bytes, cudaStream_t stream) {
+        Buf *b = nullptr;
+        for (auto &x : bufs)
+            if (cudaEventQuery(x->copied) == cudaSuccess) {
+                b = x.get();
+                break;
+            }
+        if (!b) {
+            bufs.emplace_back(new Buf());
+            b = bufs.back().get();
+            CU(cudaEventCreateWithFlags(&b->copied, cudaEventDisableTiming));
+        }
+        if (!b->pin.reserve(bytes)) return ALACB200_E_NOMEM;
+        std::memcpy(b->pin.p, src, bytes);
+        CU(cudaMemcpyAsync(dst, b->pin.p, bytes, cudaMemcpyHostToDevice, stream));
+        CU(cudaEventRecord(b->copied, stream));
+        return ALACB200_OK;
+    }
+    void release() {  // call with the device current and idle
+        for (auto &x : bufs) {
+            x->pin.release();
+            if (x->copied) cudaEventDestroy(x->copied);
+        }
+        bufs.clear();
+    }
+};
+
 // A run of packets of one track inside a pipeline chunk.
 struct Segment {
     const uint8_t *src;  // host bytes the offsets are relative to (packed packets or a whole file image)
@@ -280,6 +331,8 @@ struct Pipeline {
     uint32_t max_ctas_lat = 0;  // the same for the register-rich build that small batches run
     Slot slots[kSlots];
     uint32_t next_slot = 0;
+    DevicePathWork device_path;  // scratch of the device entry points
+    TableStaging tables;         // pinned staging of their track tables
     bool profiling = false;
     std::vector<ProfEvents> prof_events;
     alacb200_profile prof{};
@@ -316,6 +369,8 @@ struct Pipeline {
             cudaEventDestroy(pe.e1);
         }
         prof_events.clear();
+        device_path.work.release(nullptr);
+        tables.release();
         for (auto &s : slots) {
             s.work.release(s.stream);
             s.packed.release(s.stream);
@@ -519,9 +574,7 @@ struct alacb200_decoder {
     alacb200_config cfg;
     Shape shape;
     Pipeline pipe;
-    cudaStream_t device_path_stream = nullptr;  // stream device_path_work was last used (and is owned) on
-    Work device_path_work;                      // scratch of alacb200_decode_packets_device
-    PinBuf arena_in, arena_out;                 // alacb200_arena: decoder-owned pinned staging for the host wrappers
+    PinBuf arena_in, arena_out;  // alacb200_arena: decoder-owned pinned staging for the host wrappers
 };
 
 // Decoders of several tracks (any mix of cookies) on one or more devices of this process.
@@ -531,15 +584,65 @@ struct alacb200_library {
 
 namespace {
 
-// The device-path scratch is stream-ordered memory: moving to another stream first waits for the work of the previous one.
-int32_t use_device_path_stream(alacb200_decoder *dec, cudaStream_t st) {
-    if (st != dec->device_path_stream && dec->device_path_work.scratch.p) {
-        CU(cudaStreamSynchronize(dec->device_path_stream));
-        dec->device_path_work.release(dec->device_path_stream);
-    }
-    dec->device_path_stream = st;
-    return ALACB200_OK;
+size_t sample_type_bytes(int32_t sample_type) {
+    return sample_type == ALACB200_SAMPLES_S16 ? 2 : (sample_type == ALACB200_SAMPLES_S32 || sample_type == ALACB200_SAMPLES_F32) ? 4 : 0;
 }
+
+// One planar launch set on `st` for rows [row0, row0 + rows) of the packet table, all of kernel config `shape`: the decode
+// kernel into a stream-ordered intermediate (freed on the stream at the end), the frame scan of the ntracks tracks at
+// d_tracks (device), the planar pass.
+int32_t enqueue_planar(Pipeline &pipe, const Shape &shape, int32_t sample_type, const uint8_t *d_packed, const uint64_t *d_offsets,
+                       const uint32_t *d_sizes, int32_t *d_status, uint64_t *d_frame_start, const PlanarTrack *d_tracks,
+                       uint32_t ntracks, uint64_t row0, uint32_t rows, cudaStream_t st) {
+    const uint32_t ch = shape.dev.num_channels, bps = shape.dev.bps, bpf = ch * bps, fl = shape.dev.frame_length;
+    // the interleaved intermediate: packet slots of frame_bytes rounded up to 16, then out_bytes[rows]
+    const uint64_t slot = (shape.frame_bytes + 15u) / 16u * 16u;
+    uint8_t *inter = nullptr;
+    if (rows && pool_alloc((void **)&inter, (size_t)(rows * slot + (uint64_t)rows * 4u), st) != cudaSuccess) {
+        g_last_error = "cudaMallocAsync failed (planar intermediate)";
+        cudaGetLastError();
+        return ALACB200_E_NOMEM;
+    }
+    uint32_t *d_out_bytes = rows ? (uint32_t *)(inter + rows * slot) : nullptr;
+    int32_t rc = pipe.launch(pipe.device_path.work, shape, d_packed, d_offsets + row0, d_sizes + row0, rows, inter, slot, d_out_bytes,
+                             d_status + row0, st);
+    if (rc == ALACB200_OK) {
+        alac_frame_scan_kernel<<<ntracks, SCAN_THREADS, 0, st>>>(d_out_bytes, d_status, d_tracks, row0, bpf, d_frame_start);
+        if (rows) {
+            const uint32_t tile = planar_tile_frames(bpf, fl);
+            const dim3 grid(rows, (fl + tile - 1) / tile);
+            if (sample_type == ALACB200_SAMPLES_S16)
+                alac_planar_kernel<int16_t><<<grid, PLANAR_THREADS, 0, st>>>(inter, slot, d_frame_start, d_tracks, ntracks, row0, ch, bps, tile);
+            else if (sample_type == ALACB200_SAMPLES_S32)
+                alac_planar_kernel<int32_t><<<grid, PLANAR_THREADS, 0, st>>>(inter, slot, d_frame_start, d_tracks, ntracks, row0, ch, bps, tile);
+            else
+                alac_planar_kernel<float><<<grid, PLANAR_THREADS, 0, st>>>(inter, slot, d_frame_start, d_tracks, ntracks, row0, ch, bps, tile);
+        }
+        if (!cuda_ok(cudaGetLastError(), "alac_planar_kernel")) rc = ALACB200_E_CUDA;
+    }
+    if (inter) cudaFreeAsync(inter, st);
+    return rc;
+}
+
+// The track table of a planar call, uploaded through the pipeline's pinned staging into stream-ordered memory that is
+// freed on the stream after the call's launches.
+struct DeviceTracks {
+    PlanarTrack *p = nullptr;
+    int32_t upload(Pipeline &pipe, const std::vector<PlanarTrack> &host, cudaStream_t st) {
+        const size_t bytes = host.size() * sizeof(PlanarTrack);
+        if (pool_alloc((void **)&p, bytes, st) != cudaSuccess) {
+            g_last_error = "cudaMallocAsync failed (planar track table)";
+            cudaGetLastError();
+            p = nullptr;
+            return ALACB200_E_NOMEM;
+        }
+        return pipe.tables.upload(p, host.data(), bytes, st);
+    }
+    void release(cudaStream_t st) {
+        if (p) cudaFreeAsync(p, st);
+        p = nullptr;
+    }
+};
 
 // The tracks `order` on one device: already grouped by kernel config (so every launch is depth-homogeneous, SURVEY.md
 // 8e), cut into pipeline chunks that may span several tracks.
@@ -666,7 +769,6 @@ void alacb200_destroy(alacb200_decoder *dec) {
     if (!dec) return;
     DeviceGuard guard(dec->pipe.device);
     dec->pipe.destroy();  // synchronises the device first
-    dec->device_path_work.release(nullptr);
     dec->arena_in.release();
     dec->arena_out.release();
     delete dec;
@@ -703,9 +805,9 @@ int32_t alacb200_decode_packets_device(alacb200_decoder *dec, const uint8_t *d_p
     DeviceGuard guard(dec->pipe.device);
     if (!guard.ok) return ALACB200_E_CUDA;
     cudaStream_t st = (cudaStream_t)stream;
-    const int32_t rc = use_device_path_stream(dec, st);
+    const int32_t rc = dec->pipe.device_path.use(st);
     if (rc != ALACB200_OK) return rc;
-    return dec->pipe.launch(dec->device_path_work, dec->shape, d_packed, d_offsets, d_sizes, n, d_pcm_out, out_stride, d_out_bytes,
+    return dec->pipe.launch(dec->pipe.device_path.work, dec->shape, d_packed, d_offsets, d_sizes, n, d_pcm_out, out_stride, d_out_bytes,
                             d_status, st);
 }
 
@@ -715,13 +817,13 @@ int32_t alacb200_decode_planar_device(alacb200_decoder *dec, const uint8_t *d_pa
                                       void *stream) {
     (void)packed_bytes;
     if (!dec) return ALACB200_E_ARG;
-    const size_t esz = sample_type == ALACB200_SAMPLES_S16 ? 2 : (sample_type == ALACB200_SAMPLES_S32 || sample_type == ALACB200_SAMPLES_F32) ? 4 : 0;
+    const size_t esz = sample_type_bytes(sample_type);
     if (esz == 0 || (sample_type == ALACB200_SAMPLES_S16 && dec->cfg.bit_depth != 16)) {
         g_last_error = "sample_type must be S16 (16-bit streams only), S32 or F32";
         return ALACB200_E_ARG;
     }
     if (!d_frame_start) return ALACB200_E_ARG;
-    const uint32_t fl = dec->cfg.frame_length, bpf = dec->shape.dev.num_channels * dec->shape.dev.bps;
+    const uint32_t fl = dec->cfg.frame_length;
     if (n && (!d_packed || !d_offsets || !d_sizes || !d_out || !d_status)) return ALACB200_E_ARG;
     if (channel_stride < (uint64_t)n * fl || (((uintptr_t)d_out) % esz) || (((uintptr_t)d_packed) & 15u)) {
         g_last_error = "channel_stride must be >= n * frame_length; d_out aligned to its element size; d_packed 16-byte aligned";
@@ -734,33 +836,13 @@ int32_t alacb200_decode_planar_device(alacb200_decoder *dec, const uint8_t *d_pa
         CU(cudaMemsetAsync(d_frame_start, 0, sizeof(uint64_t), st));
         return ALACB200_OK;
     }
-    int32_t rc = use_device_path_stream(dec, st);
+    int32_t rc = dec->pipe.device_path.use(st);
     if (rc != ALACB200_OK) return rc;
-    // the interleaved intermediate: packet slots of frame_bytes rounded up to 16, then out_bytes[n]; freed on the stream
-    // at the end of the call
-    const uint64_t slot = (dec->shape.frame_bytes + 15u) / 16u * 16u;
-    uint8_t *inter = nullptr;
-    if (pool_alloc((void **)&inter, (size_t)(n * slot + (uint64_t)n * 4u), st) != cudaSuccess) {
-        g_last_error = "cudaMallocAsync failed (planar intermediate)";
-        cudaGetLastError();
-        return ALACB200_E_NOMEM;
-    }
-    uint32_t *d_out_bytes = (uint32_t *)(inter + n * slot);
-    rc = dec->pipe.launch(dec->device_path_work, dec->shape, d_packed, d_offsets, d_sizes, n, inter, slot, d_out_bytes, d_status, st);
-    if (rc == ALACB200_OK) {
-        alac_frame_scan_kernel<<<1, SCAN_THREADS, 0, st>>>(d_out_bytes, d_status, n, bpf, d_frame_start);
-        const uint32_t tile = planar_tile_frames(bpf, fl);
-        const dim3 grid(n, (fl + tile - 1) / tile);
-        const uint32_t ch = dec->shape.dev.num_channels, bps = dec->shape.dev.bps;
-        if (sample_type == ALACB200_SAMPLES_S16)
-            alac_planar_kernel<int16_t><<<grid, PLANAR_THREADS, 0, st>>>(inter, slot, d_frame_start, ch, bps, tile, (int16_t *)d_out, channel_stride);
-        else if (sample_type == ALACB200_SAMPLES_S32)
-            alac_planar_kernel<int32_t><<<grid, PLANAR_THREADS, 0, st>>>(inter, slot, d_frame_start, ch, bps, tile, (int32_t *)d_out, channel_stride);
-        else
-            alac_planar_kernel<float><<<grid, PLANAR_THREADS, 0, st>>>(inter, slot, d_frame_start, ch, bps, tile, (float *)d_out, channel_stride);
-        if (!cuda_ok(cudaGetLastError(), "alac_planar_kernel")) rc = ALACB200_E_CUDA;
-    }
-    cudaFreeAsync(inter, st);
+    DeviceTracks tracks;  // the one-track case of the library's planar path
+    rc = tracks.upload(dec->pipe, {PlanarTrack{0, 0, d_out, channel_stride, n, 0}}, st);
+    if (rc == ALACB200_OK)
+        rc = enqueue_planar(dec->pipe, dec->shape, sample_type, d_packed, d_offsets, d_sizes, d_status, d_frame_start, tracks.p, 1, 0, n, st);
+    tracks.release(st);
     return rc;
 }
 
@@ -933,6 +1015,104 @@ int32_t alacb200_library_decode_tracks(alacb200_library *lib, alacb200_track_des
             }
             for (uint32_t t : per_dev[d]) tracks[t].result = rcs[d];
         }
+    return rc;
+}
+
+int32_t alacb200_library_decode_planar_device(alacb200_library *lib, int device, const uint8_t *d_packed, uint64_t packed_bytes,
+                                              const uint64_t *d_offsets, const uint32_t *d_sizes, alacb200_planar_track *tracks,
+                                              uint32_t ntracks, int32_t sample_type, uint64_t *d_frame_start, int32_t *d_status,
+                                              void *stream) {
+    (void)packed_bytes;
+    if (!lib || (!tracks && ntracks) || (!d_frame_start && ntracks)) return ALACB200_E_ARG;
+    Pipeline *pipe = nullptr;
+    for (auto &p : lib->devs)
+        if (p->device == device) pipe = p.get();
+    const size_t esz = sample_type_bytes(sample_type);
+    if (!pipe || esz == 0) {
+        g_last_error = "device must be one of the library's devices; sample_type S16, S32 or F32";
+        return ALACB200_E_ARG;
+    }
+    // per track: ParseMagicCookie + NewPacketDecoder's checks (config.go:47-81, decoder.go:90-110), then the arguments
+    std::vector<Shape> shapes(ntracks);
+    uint64_t rows = 0;
+    for (uint32_t t = 0; t < ntracks; t++) {
+        alacb200_planar_track &tr = tracks[t];
+        tr.result = ALACB200_OK;
+        tr.track_status = alacb200_parse_cookie(tr.cookie, tr.cookie_len, &tr.config);
+        if (tr.track_status == ALACB200_ST_OK) tr.track_status = check_config(&tr.config);
+        rows += tr.n;
+        if (tr.track_status != ALACB200_ST_OK) {
+            tr.result = ALACB200_E_CONFIG;
+            continue;
+        }
+        shapes[t] = make_shape(tr.config, pipe->num_sms);
+        if (sample_type == ALACB200_SAMPLES_S16 && tr.config.bit_depth != 16) {
+            g_last_error = "sample_type S16 holds 16-bit streams only";
+            return ALACB200_E_ARG;
+        }
+        if (tr.n && (!tr.d_out || ((uintptr_t)tr.d_out) % esz || tr.channel_stride < (uint64_t)tr.n * tr.config.frame_length)) {
+            g_last_error = "every track's d_out must be aligned to its element size and channel_stride >= n * frame_length";
+            return ALACB200_E_ARG;
+        }
+    }
+    if (rows > UINT32_MAX) {
+        g_last_error = "more than 2^32 - 1 packets in one call";
+        return ALACB200_E_ARG;
+    }
+    if (rows && (!d_packed || !d_offsets || !d_sizes || !d_status || (((uintptr_t)d_packed) & 15u))) {
+        g_last_error = "d_packed (16-byte aligned), d_offsets, d_sizes and d_status must be set";
+        return ALACB200_E_ARG;
+    }
+    DeviceGuard guard(pipe->device);
+    if (!guard.ok) return ALACB200_E_CUDA;
+    cudaStream_t st = (cudaStream_t)stream;
+    if (rows == 0) {
+        if (ntracks) CU(cudaMemsetAsync(d_frame_start, 0, (size_t)ntracks * sizeof(uint64_t), st));
+        return ALACB200_OK;
+    }
+    int32_t rc = pipe->device_path.use(st);
+    if (rc != ALACB200_OK) return rc;
+    // the device table: the runs' tracks in order (a run: adjacent decodable tracks of one kernel config), then the tracks
+    // without a decoder
+    struct Run {
+        uint32_t first, count;  // entries of the table
+        uint32_t track;         // its first track (for the shape)
+        uint64_t row0, rows;
+    };
+    std::vector<PlanarTrack> table;
+    std::vector<Run> runs;
+    std::vector<PlanarTrack> failed;
+    uint64_t row = 0;
+    bool open = false;
+    for (uint32_t t = 0; t < ntracks; t++) {
+        const alacb200_planar_track &tr = tracks[t];
+        const PlanarTrack e{row, row + t, tr.d_out, tr.channel_stride, tr.n, tr.result == ALACB200_OK ? 0 : tr.track_status};
+        row += tr.n;
+        if (e.fail) {
+            failed.push_back(e);
+            open = false;
+            continue;
+        }
+        if (!open || !shapes[runs.back().track].same_kernel_config(shapes[t])) runs.push_back(Run{(uint32_t)table.size(), 0, t, e.row, 0});
+        open = true;
+        runs.back().count++;
+        runs.back().rows += e.n;
+        table.push_back(e);
+    }
+    const uint32_t first_failed = (uint32_t)table.size();
+    table.insert(table.end(), failed.begin(), failed.end());
+    DeviceTracks dt;
+    rc = dt.upload(*pipe, table, st);
+    for (size_t k = 0; k < runs.size() && rc == ALACB200_OK; k++) {
+        const Run &r = runs[k];
+        rc = enqueue_planar(*pipe, shapes[r.track], sample_type, d_packed, d_offsets, d_sizes, d_status, d_frame_start, dt.p + r.first,
+                            r.count, r.row0, (uint32_t)r.rows, st);
+    }
+    if (rc == ALACB200_OK && !failed.empty()) {
+        alac_frame_scan_kernel<<<(uint32_t)failed.size(), SCAN_THREADS, 0, st>>>(nullptr, d_status, dt.p + first_failed, 0, 1, d_frame_start);
+        if (!cuda_ok(cudaGetLastError(), "alac_frame_scan_kernel")) rc = ALACB200_E_CUDA;
+    }
+    dt.release(st);
     return rc;
 }
 

@@ -1,12 +1,16 @@
 // alac_planar.cuh -- channel-planar typed samples from the decode kernel's interleaved packet slots.
 //
-// alacb200_decode_planar_device runs the decode kernel into a stream-ordered intermediate of per-packet slots (stride
-// frame_bytes rounded up to 16, so every slot is 16-byte aligned) and then two passes of this file:
+// A planar launch serves a run of tracks that share one kernel config (one track for alacb200_decode_planar_device, a run
+// of adjacent tracks for alacb200_library_decode_planar_device). The rows of all tracks form one packet table, track
+// after track; a device-resident PlanarTrack per track says where its rows, frame starts and output are. The decode
+// kernel fills a stream-ordered intermediate of per-packet slots for the run's rows (stride frame_bytes rounded up to 16,
+// so every slot is 16-byte aligned), then two passes of this file run:
 //
-//   alac_frame_scan_kernel  frames[i] = out_bytes[i] / (channels * bps) (0 for a failed packet) and its exclusive prefix
-//                           sum frame_start[0..n]; one CTA, off the hot path.
-//   alac_planar_kernel      packet i, frame f, channel c -> out[c * channel_stride + frame_start[i] + f]. A CTA takes one
-//                           tile of frames of one packet: 128-bit loads stage the tile's interleaved bytes in shared
+//   alac_frame_scan_kernel  one CTA per track: frames[i] = out_bytes[i] / (channels * bps) (0 for a failed packet) and
+//                           its exclusive prefix sum, the track's frame_start[0..n]. Off the hot path.
+//   alac_planar_kernel      packet i of track t, frame f, channel c -> out_t[c * channel_stride_t + frame_start[i] + f]. A
+//                           CTA takes one tile of frames of one packet and finds the packet's track by a binary search
+//                           over the tracks' first rows: 128-bit loads stage the tile's interleaved bytes in shared
 //                           memory, then each thread converts a run of frames of one channel row and stores it, 16-byte
 //                           vector stores where the element address allows and scalar stores at the row's two ends.
 //
@@ -32,13 +36,39 @@ inline uint32_t planar_tile_frames(uint32_t frame_bytes_per_frame, uint32_t fram
     return t;
 }
 
-// One CTA: each thread owns a contiguous range of packets, sums it, the CTA scans the per-thread sums, and each thread
-// writes its range's prefixes. frame_start has n+1 entries; [n] is the total.
+// One track of a planar launch. Its rows are [row, row + n) of the shared packet table, its frame starts
+// frame_start[fs .. fs + n] (n + 1 entries, [n] is its total), and channel c of its samples starts at
+// out + c * channel_stride elements.
+struct PlanarTrack {
+    uint64_t row;
+    uint64_t fs;
+    void *out;
+    uint64_t channel_stride;
+    uint32_t n;
+    int32_t fail;  // 0, or the status word of a track without a decoder: every row gets it and every frame start is 0
+};
+
+// One CTA per track (grid = the run's tracks): each thread owns a contiguous range of the track's packets, sums it, the
+// CTA scans the per-thread sums, and each thread writes its range's prefixes. out_bytes holds the run's rows from
+// row0 on; status is the whole table.
 __global__ void __launch_bounds__(SCAN_THREADS) alac_frame_scan_kernel(const uint32_t *__restrict__ out_bytes,
-                                                                     const int32_t *__restrict__ status, uint32_t n,
+                                                                     int32_t *__restrict__ status,
+                                                                     const PlanarTrack *__restrict__ tracks, uint64_t row0,
                                                                      uint32_t bytes_per_frame,
                                                                      uint64_t *__restrict__ frame_start) {
     __shared__ uint64_t warp_sums[SCAN_THREADS / 32];
+    const PlanarTrack tr = tracks[blockIdx.x];
+    const uint32_t n = tr.n;
+    if (tr.fail) {
+        for (uint32_t i = threadIdx.x; i <= n; i += SCAN_THREADS) {
+            if (i < n) status[tr.row + i] = tr.fail;
+            frame_start[tr.fs + i] = 0;
+        }
+        return;
+    }
+    out_bytes += tr.row - row0;
+    status += tr.row;
+    frame_start += tr.fs;
     const uint32_t t = threadIdx.x, per = (n + SCAN_THREADS - 1) / SCAN_THREADS;
     const uint32_t lo = min(n, t * per), hi = min(n, lo + per);
     auto frames = [&](uint32_t i) -> uint64_t { return status[i] == 0 ? out_bytes[i] / bytes_per_frame : 0u; };
@@ -89,19 +119,33 @@ __device__ __forceinline__ int32_t planar_sample(const uint32_t *words, uint32_t
     return (int32_t)(v << drop) >> drop;
 }
 
-// grid (n packets, tiles per packet), PLANAR_THREADS threads; slots: the decode kernel's output, packet i at
-// slots + i * slot_stride (16-byte aligned); frame_start from alac_frame_scan_kernel.
+// grid (the run's rows, tiles per packet), PLANAR_THREADS threads; slots: the decode kernel's output, the run's row
+// row0 + i at slots + i * slot_stride (16-byte aligned); tracks: the run's ntracks tracks in row order; frame_start from
+// alac_frame_scan_kernel.
 template <typename T>
 __global__ void __launch_bounds__(PLANAR_THREADS) alac_planar_kernel(const uint8_t *__restrict__ slots, uint64_t slot_stride,
                                                                    const uint64_t *__restrict__ frame_start,
-                                                                   uint32_t channels, uint32_t bps, uint32_t tile_frames,
-                                                                   T *__restrict__ out,
-                                                                   uint64_t channel_stride) {
+                                                                   const PlanarTrack *__restrict__ tracks, uint32_t ntracks,
+                                                                   uint64_t row0, uint32_t channels, uint32_t bps,
+                                                                   uint32_t tile_frames) {
     constexpr uint32_t V = 16 / sizeof(T);  // elements per 16-byte store
     __shared__ uint4 tile[PLANAR_TILE_BYTES / 16 + 1];
     const uint32_t pkt = blockIdx.x;
-    const uint64_t fs = frame_start[pkt];
-    const uint32_t frames = (uint32_t)(frame_start[pkt + 1] - fs);
+    // the packet's track: the last one whose first row is at or before it (a track without rows shares its first row
+    // with the next one, so it is never picked for a row)
+    const uint64_t row = row0 + pkt;
+    uint32_t lo = 0, hi = ntracks - 1;
+    while (lo < hi) {
+        const uint32_t mid = (lo + hi + 1) / 2;
+        if (tracks[mid].row <= row) lo = mid;
+        else hi = mid - 1;
+    }
+    const PlanarTrack &tr = tracks[lo];
+    const uint64_t k0 = tr.fs + (row - tr.row);
+    T *const out = static_cast<T *>(tr.out);
+    const uint64_t channel_stride = tr.channel_stride;
+    const uint64_t fs = frame_start[k0];
+    const uint32_t frames = (uint32_t)(frame_start[k0 + 1] - fs);
     const uint32_t f0 = blockIdx.y * tile_frames;
     if (f0 >= frames) return;  // a failed or short packet: nothing in this tile
     const uint32_t cnt = min(tile_frames, frames - f0);

@@ -16,6 +16,14 @@ step by step and each call is timed with CUDA events on one stream:
 LoadTrack on the 60 s c1 M4A against what a caller does without it: NewDecoder(...).ReadAll(), unpacking the PCM into
 channel-planar samples and uploading them (host clock, median over alternating repetitions, each ending in a device
 synchronisation). The line carries the GPU's name, power limit and max SM clock, queried in the same run.
+
+`tracks`: many files in one call, for two batches of M4A images (bench.py's encoder, tests/m4a_writer.build_m4a):
+  lib     bench.build_library(0, ...): 32 tracks of 3 min of 44.1 kHz stereo, 16- and 24-bit alternating
+  clips   256 clips of 10 s of 44.1 kHz stereo, 16- and 24-bit alternating (the dataset regime)
+Per batch, arms alternating: LoadTracks against a loop of LoadTrack (host clock up to a device synchronise, float32);
+LibraryDecoder.DecodePlanar over the whole device-resident batch (ordered by config) against a loop of per-track
+PacketDecoder.DecodePlanar (one decoder per config; CUDA events on one stream); and, in a separate profiled run,
+the alac_decode_kernel* launches of one call of each.
 """
 import argparse
 import json
@@ -164,6 +172,103 @@ def load_track_leg(pkg, torch, dev, reps):
     return rec
 
 
+def tracks_leg(pkg, torch, dev, reps, steps, warmup):
+    from m4a_writer import build_m4a
+    from torch.profiler import ProfilerActivity, profile
+    threads = bench.host_cores()
+    batches = {'lib': [(wl['bits'], wl['cookie'], wl['packed'], wl['offsets'], wl['sizes'], wl['frames'])
+                       for wl in bench.build_library(0, threads)]}
+    import oracle_lib as ol
+    clips = []
+    for k in range(256):
+        bits = 16 if k % 2 == 0 else 24
+        packed, offs, sizes = bench.encode_track(bits, 2, 44100, 441000, seed=5000 + k, threads=threads, tag='clip')
+        clips.append((bits, ol.make_cookie(ol.Config.make(bit_depth=bits, num_channels=2, sample_rate=44100)), packed, offs, sizes, 441000))
+    batches['clips'] = clips
+    rec = {}
+    for name, tracks in batches.items():
+        files = []
+        for bits, cookie, packed, offs, sizes, frames in tracks:
+            packets = [bytes(packed[int(o):int(o) + int(z)]) for o, z in zip(offs, sizes)]
+            files.append(build_m4a(cookie, packets, bits=bits, last_frames=frames % 4096)[0])
+        # 1. LoadTracks vs a loop of LoadTrack
+        def one_call():
+            out = pkg.LoadTracks(files, dev)
+            torch.cuda.synchronize(dev)
+            return out
+
+        def loop():
+            out = [pkg.LoadTrack(f, dev) for f in files]
+            torch.cuda.synchronize(dev)
+            return out
+        a, b = one_call(), loop()
+        assert all(x.err is None and torch.equal(x.samples, y[0]) for x, y in zip(a, b)), 'LoadTracks differs from LoadTrack'
+        del a, b
+        t = {'load_tracks': [], 'load_track_loop': []}
+        for _ in range(reps):
+            for k, f in (('load_tracks', one_call), ('load_track_loop', loop)):
+                t0 = time.perf_counter()
+                f()
+                t[k].append((time.perf_counter() - t0) * 1e3)
+        r = {'tracks': len(files), 'packets': int(sum(len(x[4]) for x in tracks)), 'frames': int(sum(x[5] for x in tracks)),
+             'file_bytes': int(sum(len(f) for f in files)), 'reps': reps}
+        r.update({k + '_ms': float(np.median(v)) for k, v in t.items()})
+        # 2. device-resident: one library call vs per-track PacketDecoder.DecodePlanar, batch ordered by config
+        order = sorted(range(len(tracks)), key=lambda i: tracks[i][0])
+        parts, offs_all, sizes_all, base = [], [], [], 0
+        for i in order:
+            packed, offs, sizes = tracks[i][2], tracks[i][3], tracks[i][4]
+            span = (len(packed) + 15) // 16 * 16
+            parts.append(np.pad(packed, (0, span - len(packed))))
+            offs_all.append(offs.astype(np.int64) + base)
+            sizes_all.append(sizes.view(np.int32))
+            base += span
+        d_packed = torch.from_numpy(np.concatenate(parts)).to(dev)
+        d_off = torch.from_numpy(np.concatenate(offs_all)).to(dev)
+        d_sz = torch.from_numpy(np.concatenate(sizes_all)).to(dev)
+        counts = [len(tracks[i][4]) for i in order]
+        starts = np.concatenate([[0], np.cumsum(counts)])
+        cookies = [tracks[i][1] for i in order]
+        libd = pkg.NewLibraryDecoder((dev,))
+        decs = {c: pkg.NewPacketDecoder(pkg.ParseMagicCookie(c), dev) for c in set(cookies)}
+        stream = torch.cuda.Stream(dev)
+        keep = []
+
+        def lib_call():
+            with torch.cuda.stream(stream):
+                keep.append(libd.DecodePlanar(d_packed, d_off, d_sz, cookies, counts, device=dev))
+
+        def per_track():
+            with torch.cuda.stream(stream):
+                for k, c in enumerate(cookies):
+                    a, b = int(starts[k]), int(starts[k + 1])
+                    keep.append(decs[c].DecodePlanar(d_packed, d_off[a:b], d_sz[a:b]))
+
+        def drop(f):
+            def g():
+                f()
+                keep.clear()  # the caching allocator reuses the outputs on the same stream
+            return g
+        ms = time_arms(torch, stream, {'library_decode_planar': drop(lib_call), 'per_track_decode_planar': drop(per_track)}, steps, warmup)
+        r.update({k + '_ms': float(np.median(v)) for k, v in ms.items()})
+        # 3. decode launches per call, in a separate profiled run
+        def launches(f):
+            torch.cuda.synchronize(dev)
+            with profile(activities=[ProfilerActivity.CUDA]) as prof:
+                f()
+                torch.cuda.synchronize(dev)
+            return sum('alac_decode_kernel' in e.name for e in prof.events() if e.device_type == torch.autograd.DeviceType.CUDA)
+        r['decode_launches'] = {'load_tracks': launches(one_call), 'load_track_loop': launches(loop),
+                                'library_decode_planar': launches(drop(lib_call)), 'per_track_decode_planar': launches(drop(per_track))}
+        for d in decs.values():
+            d.close()
+        libd.close()
+        del d_packed, d_off, d_sz
+        torch.cuda.empty_cache()
+        rec[name] = r
+    return rec
+
+
 def main():
     ap = argparse.ArgumentParser(description=__doc__.split('\n')[0])
     ap.add_argument('--steps', type=int, default=20)
@@ -171,6 +276,7 @@ def main():
     ap.add_argument('--reps', type=int, default=20, help='repetitions of each LoadTrack arm')
     ap.add_argument('--workloads', default='c1,c2,c3,c4')
     ap.add_argument('--device', type=int, default=0)
+    ap.add_argument('--tracks-only', action='store_true', help='only the `tracks` record')
     args = ap.parse_args()
     if args.steps < 1:
         ap.error('--steps must be >= 1')
@@ -184,10 +290,12 @@ def main():
     peak, peak_src = bench.measured_peak_gbs()
     line = {'tool': 'tools/planar_bench.py', 'gpu': gpu_info(dev), 'steps': args.steps, 'warmup': args.warmup,
             'peak_gbs': peak, 'peak_source': peak_src, 'workloads': {}}
-    for name in args.workloads.split(','):
-        wl = bench.build_workload(name, seed=SEEDS[name], threads=bench.host_cores())
-        line['workloads'][name] = planar_workload(pkg, torch, dev, wl, args.steps, args.warmup, peak)
-    line['load_track'] = load_track_leg(pkg, torch, dev, args.reps)
+    if not args.tracks_only:
+        for name in args.workloads.split(','):
+            wl = bench.build_workload(name, seed=SEEDS[name], threads=bench.host_cores())
+            line['workloads'][name] = planar_workload(pkg, torch, dev, wl, args.steps, args.warmup, peak)
+        line['load_track'] = load_track_leg(pkg, torch, dev, args.reps)
+    line['tracks'] = tracks_leg(pkg, torch, dev, args.reps, args.steps, args.warmup)
     print(json.dumps(line))
 
 
