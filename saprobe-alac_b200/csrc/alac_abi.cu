@@ -14,6 +14,7 @@
 #include <mutex>
 #include <string>
 #include <thread>
+#include <tuple>
 #include <vector>
 
 #include "../../include/alac_b200.h"
@@ -300,14 +301,24 @@ int32_t check_config(const alacb200_config *cfg) {
     return ALACB200_ST_OK;
 }
 
+// ParseMagicCookie + NewPacketDecoder's checks (config.go:47-81, decoder.go:90-110): parses `cookie` into `config` and
+// returns ALACB200_ST_OK or why the track has no decoder.
+int32_t admit_cookie(const uint8_t *cookie, size_t cookie_len, alacb200_config *config) {
+    const int32_t st = alacb200_parse_cookie(cookie, cookie_len, config);
+    return st == ALACB200_ST_OK ? check_config(config) : st;
+}
+
+uint64_t packet_pcm_bytes(const alacb200_config &cfg) {
+    return (uint64_t)cfg.frame_length * cfg.num_channels * (uint32_t)alacb200_bytes_per_sample(cfg.bit_depth);
+}
+
 // The part of a cookie the kernel needs, and the size of a decoded packet.
 struct Shape {
     DevConfig dev;
     uint64_t frame_bytes;
-    bool same_kernel_config(const Shape &o) const {
-        return dev.frame_length == o.dev.frame_length && dev.bit_depth == o.dev.bit_depth && dev.num_channels == o.dev.num_channels &&
-               dev.pb == o.dev.pb && dev.mb == o.dev.mb && dev.kb == o.dev.kb;
-    }
+    // The fields that make a kernel config, in the order tracks are sorted by: a launch never mixes two configs.
+    auto kernel_config() const { return std::tie(dev.bit_depth, dev.num_channels, dev.frame_length, dev.pb, dev.mb, dev.kb); }
+    bool same_kernel_config(const Shape &o) const { return kernel_config() == o.kernel_config(); }
 };
 Shape make_shape(const alacb200_config &cfg, uint32_t num_sms) {
     Shape s;
@@ -319,7 +330,7 @@ Shape make_shape(const alacb200_config &cfg, uint32_t num_sms) {
     s.dev.mb = cfg.mb;
     s.dev.kb = cfg.kb;
     s.dev.num_sms = num_sms;
-    s.frame_bytes = (uint64_t)cfg.frame_length * cfg.num_channels * s.dev.bps;
+    s.frame_bytes = packet_pcm_bytes(cfg);
     return s;
 }
 
@@ -624,25 +635,105 @@ int32_t enqueue_planar(Pipeline &pipe, const Shape &shape, int32_t sample_type, 
     return rc;
 }
 
-// The track table of a planar call, uploaded through the pipeline's pinned staging into stream-ordered memory that is
-// freed on the stream after the call's launches.
-struct DeviceTracks {
-    PlanarTrack *p = nullptr;
-    int32_t upload(Pipeline &pipe, const std::vector<PlanarTrack> &host, cudaStream_t st) {
-        const size_t bytes = host.size() * sizeof(PlanarTrack);
-        if (pool_alloc((void **)&p, bytes, st) != cudaSuccess) {
-            g_last_error = "cudaMallocAsync failed (planar track table)";
-            cudaGetLastError();
-            p = nullptr;
-            return ALACB200_E_NOMEM;
-        }
-        return pipe.tables.upload(p, host.data(), bytes, st);
-    }
-    void release(cudaStream_t st) {
-        if (p) cudaFreeAsync(p, st);
-        p = nullptr;
-    }
+// A track of a planar call. fail: ALACB200_ST_OK, or the status word of a track whose cookie was not admitted (its shape
+// is then unset and its arguments are not checked).
+struct PlanarInput {
+    Shape shape;
+    uint32_t n;  // its rows of the shared packet table, which holds the tracks' rows in track order
+    void *d_out;
+    uint64_t channel_stride;
+    int32_t fail;
 };
+
+// The planar path of both planar entry points, on `st`. Argument errors fail the whole call before anything is enqueued.
+// Then every maximal run of adjacent admitted tracks of one kernel config is one enqueue_planar, and one frame scan over
+// the tracks that were not admitted writes their status word to their rows and zeros to their frame starts.
+int32_t decode_planar_on(Pipeline &pipe, const std::vector<PlanarInput> &tracks, int32_t sample_type, const uint8_t *d_packed,
+                         const uint64_t *d_offsets, const uint32_t *d_sizes, uint64_t *d_frame_start, int32_t *d_status,
+                         cudaStream_t st) {
+    const size_t esz = sample_type_bytes(sample_type);
+    if (esz == 0 || (!d_frame_start && !tracks.empty())) {
+        g_last_error = "sample_type must be S16, S32 or F32; d_frame_start must be set";
+        return ALACB200_E_ARG;
+    }
+    uint64_t rows = 0;
+    for (const PlanarInput &tr : tracks) {
+        rows += tr.n;
+        if (tr.fail) continue;
+        if (sample_type == ALACB200_SAMPLES_S16 && tr.shape.dev.bit_depth != 16) {
+            g_last_error = "sample_type S16 holds 16-bit streams only";
+            return ALACB200_E_ARG;
+        }
+        if (tr.n && (!tr.d_out || ((uintptr_t)tr.d_out) % esz || tr.channel_stride < (uint64_t)tr.n * tr.shape.dev.frame_length)) {
+            g_last_error = "every track's d_out must be aligned to its element size and channel_stride >= n * frame_length";
+            return ALACB200_E_ARG;
+        }
+    }
+    if (rows > UINT32_MAX) {
+        g_last_error = "more than 2^32 - 1 packets in one call";
+        return ALACB200_E_ARG;
+    }
+    if (rows && (!d_packed || !d_offsets || !d_sizes || !d_status || (((uintptr_t)d_packed) & 15u))) {
+        g_last_error = "d_packed (16-byte aligned), d_offsets, d_sizes and d_status must be set";
+        return ALACB200_E_ARG;
+    }
+    DeviceGuard guard(pipe.device);
+    if (!guard.ok) return ALACB200_E_CUDA;
+    if (rows == 0) {
+        if (!tracks.empty()) CU(cudaMemsetAsync(d_frame_start, 0, tracks.size() * sizeof(uint64_t), st));
+        return ALACB200_OK;
+    }
+    int32_t rc = pipe.device_path.use(st);
+    if (rc != ALACB200_OK) return rc;
+    // the device table: the runs' tracks in order, then the tracks that were not admitted
+    struct Run {
+        uint32_t first, count;  // entries of the table
+        uint32_t track;         // its first track (for the shape)
+        uint64_t row0, rows;
+    };
+    std::vector<PlanarTrack> table;
+    std::vector<Run> runs;
+    std::vector<PlanarTrack> failed;
+    uint64_t row = 0;
+    bool open = false;
+    for (uint32_t t = 0; t < tracks.size(); t++) {
+        const PlanarInput &tr = tracks[t];
+        const PlanarTrack e{row, row + t, tr.d_out, tr.channel_stride, tr.n, tr.fail};
+        row += tr.n;
+        if (e.fail) {
+            failed.push_back(e);
+            open = false;
+            continue;
+        }
+        if (!open || !tracks[runs.back().track].shape.same_kernel_config(tr.shape)) runs.push_back(Run{(uint32_t)table.size(), 0, t, e.row, 0});
+        open = true;
+        runs.back().count++;
+        runs.back().rows += e.n;
+        table.push_back(e);
+    }
+    const uint32_t first_failed = (uint32_t)table.size();
+    table.insert(table.end(), failed.begin(), failed.end());
+    // uploaded through the pipeline's pinned staging into stream-ordered memory that is freed on the stream after the launches
+    const size_t table_bytes = table.size() * sizeof(PlanarTrack);
+    PlanarTrack *d_table = nullptr;
+    if (pool_alloc((void **)&d_table, table_bytes, st) != cudaSuccess) {
+        g_last_error = "cudaMallocAsync failed (planar track table)";
+        cudaGetLastError();
+        return ALACB200_E_NOMEM;
+    }
+    rc = pipe.tables.upload(d_table, table.data(), table_bytes, st);
+    for (size_t k = 0; k < runs.size() && rc == ALACB200_OK; k++) {
+        const Run &r = runs[k];
+        rc = enqueue_planar(pipe, tracks[r.track].shape, sample_type, d_packed, d_offsets, d_sizes, d_status, d_frame_start,
+                            d_table + r.first, r.count, r.row0, (uint32_t)r.rows, st);
+    }
+    if (rc == ALACB200_OK && !failed.empty()) {
+        alac_frame_scan_kernel<<<(uint32_t)failed.size(), SCAN_THREADS, 0, st>>>(nullptr, d_status, d_table + first_failed, 0, 1, d_frame_start);
+        if (!cuda_ok(cudaGetLastError(), "alac_frame_scan_kernel")) rc = ALACB200_E_CUDA;
+    }
+    cudaFreeAsync(d_table, st);
+    return rc;
+}
 
 // The tracks `order` on one device: already grouped by kernel config (so every launch is depth-homogeneous, SURVEY.md
 // 8e), cut into pipeline chunks that may span several tracks.
@@ -817,33 +908,14 @@ int32_t alacb200_decode_planar_device(alacb200_decoder *dec, const uint8_t *d_pa
                                       void *stream) {
     (void)packed_bytes;
     if (!dec) return ALACB200_E_ARG;
+    // unlike a track of the library form, d_out and d_packed must be aligned even when there are no packets
     const size_t esz = sample_type_bytes(sample_type);
-    if (esz == 0 || (sample_type == ALACB200_SAMPLES_S16 && dec->cfg.bit_depth != 16)) {
-        g_last_error = "sample_type must be S16 (16-bit streams only), S32 or F32";
+    if (n == 0 && ((esz && ((uintptr_t)d_out) % esz) || (((uintptr_t)d_packed) & 15u))) {
+        g_last_error = "d_out must be aligned to its element size; d_packed 16-byte aligned";
         return ALACB200_E_ARG;
     }
-    if (!d_frame_start) return ALACB200_E_ARG;
-    const uint32_t fl = dec->cfg.frame_length;
-    if (n && (!d_packed || !d_offsets || !d_sizes || !d_out || !d_status)) return ALACB200_E_ARG;
-    if (channel_stride < (uint64_t)n * fl || (((uintptr_t)d_out) % esz) || (((uintptr_t)d_packed) & 15u)) {
-        g_last_error = "channel_stride must be >= n * frame_length; d_out aligned to its element size; d_packed 16-byte aligned";
-        return ALACB200_E_ARG;
-    }
-    DeviceGuard guard(dec->pipe.device);
-    if (!guard.ok) return ALACB200_E_CUDA;
-    cudaStream_t st = (cudaStream_t)stream;
-    if (n == 0) {
-        CU(cudaMemsetAsync(d_frame_start, 0, sizeof(uint64_t), st));
-        return ALACB200_OK;
-    }
-    int32_t rc = dec->pipe.device_path.use(st);
-    if (rc != ALACB200_OK) return rc;
-    DeviceTracks tracks;  // the one-track case of the library's planar path
-    rc = tracks.upload(dec->pipe, {PlanarTrack{0, 0, d_out, channel_stride, n, 0}}, st);
-    if (rc == ALACB200_OK)
-        rc = enqueue_planar(dec->pipe, dec->shape, sample_type, d_packed, d_offsets, d_sizes, d_status, d_frame_start, tracks.p, 1, 0, n, st);
-    tracks.release(st);
-    return rc;
+    return decode_planar_on(dec->pipe, {PlanarInput{dec->shape, n, d_out, channel_stride, ALACB200_ST_OK}}, sample_type, d_packed,
+                            d_offsets, d_sizes, d_frame_start, d_status, (cudaStream_t)stream);
 }
 
 int32_t alacb200_decode_packets(alacb200_decoder *dec, const uint8_t *packed, uint64_t packed_bytes, const uint64_t *offsets,
@@ -945,23 +1017,19 @@ int32_t alacb200_library_devices(const alacb200_library *lib) { return lib ? (in
 
 int32_t alacb200_library_decode_tracks(alacb200_library *lib, alacb200_track_desc *tracks, uint32_t ntracks) {
     if (!lib || (!tracks && ntracks)) return ALACB200_E_ARG;
-    // per track: ParseMagicCookie + NewPacketDecoder's checks (config.go:47-81, decoder.go:90-110)
-    std::vector<Shape> shapes(ntracks);
     std::vector<uint64_t> weight(ntracks, 0);
     std::vector<uint32_t> good;
     for (uint32_t t = 0; t < ntracks; t++) {
         alacb200_track_desc &tr = tracks[t];
         tr.result = ALACB200_OK;
         tr.device = -1;
-        tr.track_status = alacb200_parse_cookie(tr.cookie, tr.cookie_len, &tr.config);
-        if (tr.track_status == ALACB200_ST_OK) tr.track_status = check_config(&tr.config);
+        tr.track_status = admit_cookie(tr.cookie, tr.cookie_len, &tr.config);
         if (tr.track_status != ALACB200_ST_OK) {
             tr.result = ALACB200_E_CONFIG;
             continue;
         }
-        shapes[t] = make_shape(tr.config, 0);
         if (tr.n == 0) continue;
-        if (!tr.data || !tr.offsets || !tr.sizes || !tr.pcm_out || !tr.out_bytes || !tr.status || !stride_ok(tr.out_stride, shapes[t].frame_bytes)) {
+        if (!tr.data || !tr.offsets || !tr.sizes || !tr.pcm_out || !tr.out_bytes || !tr.status || !stride_ok(tr.out_stride, packet_pcm_bytes(tr.config))) {
             tr.result = ALACB200_E_ARG;
             continue;
         }
@@ -973,26 +1041,18 @@ int32_t alacb200_library_decode_tracks(alacb200_library *lib, alacb200_track_des
     uint64_t total = 0;
     for (uint32_t t : good) total += weight[t];
     std::vector<std::vector<uint32_t>> per_dev(nd);
+    std::vector<Shape> shapes(ntracks);
     uint64_t acc = 0;
     for (uint32_t t : good) {
         size_t d = total ? (size_t)(((long double)acc + weight[t] / 2.0L) * nd / (long double)total) : 0;
         d = std::min(d, nd - 1);
         per_dev[d].push_back(t);
         tracks[t].device = lib->devs[d]->device;
+        shapes[t] = make_shape(tracks[t].config, lib->devs[d]->num_sms);
         acc += weight[t];
     }
-    for (size_t d = 0; d < nd; d++) {
-        for (uint32_t t : per_dev[d]) shapes[t].dev.num_sms = lib->devs[d]->num_sms;
-        std::stable_sort(per_dev[d].begin(), per_dev[d].end(), [&](uint32_t a, uint32_t b) {
-            const DevConfig &x = shapes[a].dev, &y = shapes[b].dev;
-            if (x.bit_depth != y.bit_depth) return x.bit_depth < y.bit_depth;
-            if (x.num_channels != y.num_channels) return x.num_channels < y.num_channels;
-            if (x.frame_length != y.frame_length) return x.frame_length < y.frame_length;
-            if (x.pb != y.pb) return x.pb < y.pb;
-            if (x.mb != y.mb) return x.mb < y.mb;
-            return x.kb < y.kb;
-        });
-    }
+    for (auto &order : per_dev)
+        std::stable_sort(order.begin(), order.end(), [&](uint32_t a, uint32_t b) { return shapes[a].kernel_config() < shapes[b].kernel_config(); });
     std::vector<int32_t> rcs(nd, ALACB200_OK);
     std::vector<std::string> errs(nd);
     auto run = [&](size_t d) {
@@ -1023,97 +1083,23 @@ int32_t alacb200_library_decode_planar_device(alacb200_library *lib, int device,
                                               uint32_t ntracks, int32_t sample_type, uint64_t *d_frame_start, int32_t *d_status,
                                               void *stream) {
     (void)packed_bytes;
-    if (!lib || (!tracks && ntracks) || (!d_frame_start && ntracks)) return ALACB200_E_ARG;
+    if (!lib || (!tracks && ntracks)) return ALACB200_E_ARG;
     Pipeline *pipe = nullptr;
     for (auto &p : lib->devs)
         if (p->device == device) pipe = p.get();
-    const size_t esz = sample_type_bytes(sample_type);
-    if (!pipe || esz == 0) {
-        g_last_error = "device must be one of the library's devices; sample_type S16, S32 or F32";
+    if (!pipe) {
+        g_last_error = "device must be one of the library's devices";
         return ALACB200_E_ARG;
     }
-    // per track: ParseMagicCookie + NewPacketDecoder's checks (config.go:47-81, decoder.go:90-110), then the arguments
-    std::vector<Shape> shapes(ntracks);
-    uint64_t rows = 0;
+    std::vector<PlanarInput> in(ntracks);
     for (uint32_t t = 0; t < ntracks; t++) {
         alacb200_planar_track &tr = tracks[t];
-        tr.result = ALACB200_OK;
-        tr.track_status = alacb200_parse_cookie(tr.cookie, tr.cookie_len, &tr.config);
-        if (tr.track_status == ALACB200_ST_OK) tr.track_status = check_config(&tr.config);
-        rows += tr.n;
-        if (tr.track_status != ALACB200_ST_OK) {
-            tr.result = ALACB200_E_CONFIG;
-            continue;
-        }
-        shapes[t] = make_shape(tr.config, pipe->num_sms);
-        if (sample_type == ALACB200_SAMPLES_S16 && tr.config.bit_depth != 16) {
-            g_last_error = "sample_type S16 holds 16-bit streams only";
-            return ALACB200_E_ARG;
-        }
-        if (tr.n && (!tr.d_out || ((uintptr_t)tr.d_out) % esz || tr.channel_stride < (uint64_t)tr.n * tr.config.frame_length)) {
-            g_last_error = "every track's d_out must be aligned to its element size and channel_stride >= n * frame_length";
-            return ALACB200_E_ARG;
-        }
+        tr.track_status = admit_cookie(tr.cookie, tr.cookie_len, &tr.config);
+        tr.result = tr.track_status == ALACB200_ST_OK ? ALACB200_OK : ALACB200_E_CONFIG;
+        const Shape shape = tr.result == ALACB200_OK ? make_shape(tr.config, pipe->num_sms) : Shape{};
+        in[t] = PlanarInput{shape, tr.n, tr.d_out, tr.channel_stride, tr.track_status};
     }
-    if (rows > UINT32_MAX) {
-        g_last_error = "more than 2^32 - 1 packets in one call";
-        return ALACB200_E_ARG;
-    }
-    if (rows && (!d_packed || !d_offsets || !d_sizes || !d_status || (((uintptr_t)d_packed) & 15u))) {
-        g_last_error = "d_packed (16-byte aligned), d_offsets, d_sizes and d_status must be set";
-        return ALACB200_E_ARG;
-    }
-    DeviceGuard guard(pipe->device);
-    if (!guard.ok) return ALACB200_E_CUDA;
-    cudaStream_t st = (cudaStream_t)stream;
-    if (rows == 0) {
-        if (ntracks) CU(cudaMemsetAsync(d_frame_start, 0, (size_t)ntracks * sizeof(uint64_t), st));
-        return ALACB200_OK;
-    }
-    int32_t rc = pipe->device_path.use(st);
-    if (rc != ALACB200_OK) return rc;
-    // the device table: the runs' tracks in order (a run: adjacent decodable tracks of one kernel config), then the tracks
-    // without a decoder
-    struct Run {
-        uint32_t first, count;  // entries of the table
-        uint32_t track;         // its first track (for the shape)
-        uint64_t row0, rows;
-    };
-    std::vector<PlanarTrack> table;
-    std::vector<Run> runs;
-    std::vector<PlanarTrack> failed;
-    uint64_t row = 0;
-    bool open = false;
-    for (uint32_t t = 0; t < ntracks; t++) {
-        const alacb200_planar_track &tr = tracks[t];
-        const PlanarTrack e{row, row + t, tr.d_out, tr.channel_stride, tr.n, tr.result == ALACB200_OK ? 0 : tr.track_status};
-        row += tr.n;
-        if (e.fail) {
-            failed.push_back(e);
-            open = false;
-            continue;
-        }
-        if (!open || !shapes[runs.back().track].same_kernel_config(shapes[t])) runs.push_back(Run{(uint32_t)table.size(), 0, t, e.row, 0});
-        open = true;
-        runs.back().count++;
-        runs.back().rows += e.n;
-        table.push_back(e);
-    }
-    const uint32_t first_failed = (uint32_t)table.size();
-    table.insert(table.end(), failed.begin(), failed.end());
-    DeviceTracks dt;
-    rc = dt.upload(*pipe, table, st);
-    for (size_t k = 0; k < runs.size() && rc == ALACB200_OK; k++) {
-        const Run &r = runs[k];
-        rc = enqueue_planar(*pipe, shapes[r.track], sample_type, d_packed, d_offsets, d_sizes, d_status, d_frame_start, dt.p + r.first,
-                            r.count, r.row0, (uint32_t)r.rows, st);
-    }
-    if (rc == ALACB200_OK && !failed.empty()) {
-        alac_frame_scan_kernel<<<(uint32_t)failed.size(), SCAN_THREADS, 0, st>>>(nullptr, d_status, dt.p + first_failed, 0, 1, d_frame_start);
-        if (!cuda_ok(cudaGetLastError(), "alac_frame_scan_kernel")) rc = ALACB200_E_CUDA;
-    }
-    dt.release(st);
-    return rc;
+    return decode_planar_on(*pipe, in, sample_type, d_packed, d_offsets, d_sizes, d_frame_start, d_status, (cudaStream_t)stream);
 }
 
 // The public pinned allocator goes through the same pool; the capacity of a block is kept in a small table.
